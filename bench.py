@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference's algorithm on host cores
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as .npy
 
 Workload (BASELINE.json configs[1], SURVEY.md section 8d "cfg 2"): random-action step throughput,
 vs_dummy / hard difficulty, max_episode_steps=500, `--envs-per-gpu` envs per GPU (default
@@ -59,7 +60,15 @@ def parse_args():
     ap.add_argument("--ppo-envs4", type=int, default=1 << 20, help="envs per GPU of the sharded vs_dummy PPO run (configs[4])")
     ap.add_argument("--ppo-samples", type=int, default=1 << 21, help="samples per GPU per PPO iteration (rollout_steps = this / envs)")
     ap.add_argument("--ppo-iters", type=int, default=3, help="PPO iterations per run (the first one is warm-up)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (a fixed sample of "
+                         "the envs), so that two builds can be compared output for output; bench_outputs/ is git-ignored")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 arm; it does not apply to --impl reference")
+    return args
 
 
 def measured_peaks():
@@ -367,11 +376,11 @@ def reference_arm(args):
         return 0
     W = min(max(args.warmup, 3), 50)
     # the CPU arm has no caches or clocks to settle: its warm-up is capped, and each "step" is one
-    # MultiEnvRunner.step over a bounded sample of the workload's envs (64 per host core)
-    steps = min(args.steps, 400)
-    ref = run_reference_processes(args, W, steps)
+    # MultiEnvRunner.step over a bounded sample of the workload's envs (64 per host core). Both legs
+    # time exactly --steps steps.
+    ref = run_reference_processes(args, W, args.steps)
     n = args.cpu_sample_envs
-    port = run_oracle(args, n, args.steps, W, budget_s=20.0 if ref else 150.0)
+    port = run_oracle(args, n, args.steps, W)
     port_line = {"value": port["value"], "unit": UNIT, "cores": port["cores"], "kind": "port",
                  "sample": f"{n} envs x {port['steps']} steps through oracle/inversus_oracle.c (the C restatement), "
                            f"fp32 obs written every step, auto-reset, {port['cores']} pthreads"}
@@ -429,6 +438,36 @@ def time_steps(sim, torch, acts, acts2, steps, first_t=0):
         ev[t + 1].record()
     torch.cuda.synchronize()
     return [ev[i].elapsed_time(ev[i + 1]) for i in range(steps)], ev[0].elapsed_time(ev[steps])
+
+
+DUMP_ENVS = 1 << 18      # envs whose per-env outputs are written (all of them up to this many)
+DUMP_OBS_ENVS = 2048     # of those, envs whose observations are written (7.2 KB per view in fp32)
+DUMP_SAMPLE_SEED = 12345
+
+
+def dump_outputs(path, sim):
+    """Writes what the last `sim.step` returned -- (obs, extra), reward, done, info, plus the episode
+    statistics it leaves as attributes and, in selfplay, P2's view (obs_p2, extra_p2) -- as
+    float32/float64 .npy files, for a fixed, seeded sample of the envs: at most about 47 MB whatever
+    the env count and mode. env_index / obs_env_index name the sampled envs."""
+    import numpy as np
+    import torch
+    pick = np.random.RandomState(DUMP_SAMPLE_SEED).permutation(sim.num_envs)[:DUMP_ENVS]
+    rows, obs_rows = np.sort(pick), np.sort(pick[:DUMP_OBS_ENVS])
+    idx = torch.from_numpy(rows).to(sim.device)
+    obs_idx = torch.from_numpy(obs_rows).to(sim.device)
+    arrays = {"env_index": rows.astype(np.float64), "obs_env_index": obs_rows.astype(np.float64)}
+    outputs = [("obs", sim.obs, obs_idx, torch.float32), ("extra", sim.extra, idx, torch.float32),
+               ("reward", sim.reward, idx, torch.float32), ("done", sim.done, idx, torch.float32),
+               ("info", sim.info, idx, torch.float32), ("episode_steps", sim.episode_steps, idx, torch.float64),
+               ("episode_return", sim.episode_return, idx, torch.float64)]
+    if sim.obs_p2 is not None:
+        outputs += [("obs_p2", sim.obs_p2, obs_idx, torch.float32), ("extra_p2", sim.extra_p2, idx, torch.float32)]
+    for name, t, ix, dt in outputs:
+        arrays[name] = t.index_select(0, ix).to(dt).cpu().numpy()
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
 
 
 _REAL_STDOUT = None
@@ -511,6 +550,8 @@ def main():
     launches = sim.launch_count - launches0
     status = sim.poll_status()
     assert status == 0, f"device status bits {status}"
+    if args.dump_outputs and rank == 0:  # before the e2e leg steps the same envs again
+        dump_outputs(args.dump_outputs, sim)
     t = torch.tensor([total_ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

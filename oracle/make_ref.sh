@@ -1,14 +1,14 @@
 #!/bin/sh
 # oracle/make_ref.sh -- stage the UNMODIFIED reference step loop under oracle/_ref/ so that the CPU
 # legs of bench.py can time the reference itself (kind "reference") instead of the restatement in
-# oracle/py_loop.py. Run in the builder container, where /root/reference exists; oracle/_ref/ is
-# git-ignored (never part of the history) but travels to the GPU box with the snapshot, like the
-# built .so files. Only the pure-Python files of the step path are staged: the engine package and
+# oracle/py_loop.py. Usage: make_ref.sh <checkout of the original project> (default
+# $INVERSUS_REFERENCE_ROOT); oracle/_ref/ is git-ignored, like the built .so files.
+# Only the pure-Python files of the step path are staged: the engine package and
 # the wrapper module (numpy + stdlib only). Nothing in the product imports it
 # (tests/test_capi_surface.py::test_product_never_imports_the_oracle).
 set -e
 HERE="$(cd "$(dirname "$0")" && pwd)"
-REF="${1:-/root/reference}"
+REF="${1:-$INVERSUS_REFERENCE_ROOT}"
 if [ ! -d "$REF/inversus" ] || [ ! -f "$REF/inversus_rl/env_wrappers.py" ]; then
     echo "make_ref: no reference at $REF (nothing staged)"; exit 0
 fi

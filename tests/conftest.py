@@ -14,4 +14,4 @@ for p in (ROOT, os.path.join(ROOT, "tests")):
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (B200); run with -m gpu")
-    config.addinivalue_line("markers", "live_reference: needs /root/reference (builder container only)")
+    config.addinivalue_line("markers", "live_reference: needs INVERSUS_REFERENCE_ROOT, a checkout of the original project")

@@ -1,12 +1,17 @@
 """Golden vectors for GAE from the LIVE reference PPOAgent.compute_advantages
-(inversus_rl/ppo_agent.py:127-157). Builder-container only. Writes tests/golden/gae_reference.npz."""
+(inversus_rl/ppo_agent.py:127-157). Needs a checkout of the original project:
+    INVERSUS_REFERENCE_ROOT=<checkout> python tests/golden/make_gae_golden.py
+Writes tests/golden/gae_reference.npz."""
 import os
 import sys
 
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-sys.path.insert(0, "/root/reference")
+sys.path.insert(0, os.path.dirname(HERE))
+from ref_harness import import_reference  # noqa: E402
+
+import_reference()
 from inversus_rl.ppo_agent import PPOAgent  # noqa: E402
 import torch.nn as nn  # noqa: E402
 

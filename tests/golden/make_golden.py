@@ -1,7 +1,7 @@
 """Generate tests/golden/*.npz by running the LIVE Python reference with injected draws.
 
-Run in the builder container only (needs /root/reference):
-    python tests/golden/make_golden.py
+Needs a checkout of the original project:
+    INVERSUS_REFERENCE_ROOT=<checkout> python tests/golden/make_golden.py
 The fixtures are the reference's own outputs; oracle/ and the CUDA path are both checked
 against them (tests/test_oracle_golden.py, tests/test_cuda_parity.py).
 """
@@ -46,7 +46,7 @@ class ReferenceBackend:
 
 
 def main():
-    assert reference_available(), "needs /root/reference"
+    assert reference_available(), "set INVERSUS_REFERENCE_ROOT to a checkout of the original project"
     only = sys.argv[1:]
     for name, sc in SCENARIOS.items():
         if only and name not in only:

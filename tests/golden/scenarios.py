@@ -18,7 +18,9 @@ TABLE_STRIDE = 64
 
 SCENARIOS = {
     # name: mode, difficulty, max_episode_steps, n_envs, steps, seed, action mix, draw source, reset policy
-    "hard_auto":   dict(mode="dummy", difficulty="hard", max_steps=500, n=40, T=620, seed=11, actions="uniform", draws="philox", resets="auto"),
+    # hard_auto holds the first 480 steps of a 620-step recording (no episode of it reaches the
+    # timeout), which keeps the fixture under 1 MB; step t's actions do not depend on the step count
+    "hard_auto":   dict(mode="dummy", difficulty="hard", max_steps=500, n=40, T=480, seed=11, actions="uniform", draws="philox", resets="auto"),
     "easy_auto":   dict(mode="dummy", difficulty="easy", max_steps=500, n=24, T=540, seed=12, actions="uniform", draws="philox", resets="auto"),
     "hard_charge": dict(mode="dummy", difficulty="hard", max_steps=500, n=32, T=300, seed=13, actions="charge", draws="philox", resets="auto"),
     "selfplay":    dict(mode="selfplay", difficulty="hard", max_steps=500, n=40, T=400, seed=14, actions="uniform", draws="philox", resets="auto"),

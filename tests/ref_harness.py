@@ -1,7 +1,8 @@
-"""Drives the LIVE Python reference (/root/reference) with injected draws.
+"""Drives the LIVE Python reference with injected draws.
 
-Builder-container only: /root/reference does not exist on the GPU box. Used by
-tests/golden/make_golden.py (fixture generation) and tests/test_oracle_vs_reference_live.py
+The reference is a checkout of the original project (Jason-Hoford/inversus-reinforcement-learning),
+named by the environment variable INVERSUS_REFERENCE_ROOT; it is not part of this repository. Used
+by tests/golden/make_golden.py (fixture generation) and tests/test_oracle_vs_reference_live.py
 (differential fuzz, skipped when the reference is absent). Never imported by the product,
 bench.py or any -m gpu test.
 
@@ -19,7 +20,8 @@ import sys
 
 import numpy as np
 
-REFERENCE_ROOT = os.environ.get("INVERSUS_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("INVERSUS_REFERENCE_ROOT", "")
+SKIP_REASON = "original project not present (set INVERSUS_REFERENCE_ROOT to a checkout of it)"
 STREAM_RESET = 0xFFFFFFFF
 TABLE_STRIDE = 64
 TABLE_RESET_OFF = 16
@@ -27,7 +29,7 @@ M32 = 0xFFFFFFFF
 
 
 def reference_available() -> bool:
-    return os.path.isdir(os.path.join(REFERENCE_ROOT, "inversus_rl"))
+    return bool(REFERENCE_ROOT) and os.path.isdir(os.path.join(REFERENCE_ROOT, "inversus_rl"))
 
 
 def philox4x32_10(ctr, key):
@@ -90,6 +92,8 @@ class DrawShim:
 
 
 def import_reference():
+    if not reference_available():
+        raise RuntimeError(SKIP_REASON)
     if REFERENCE_ROOT not in sys.path:
         sys.path.insert(0, REFERENCE_ROOT)
     import inversus.core  # noqa: F401

@@ -1,6 +1,6 @@
 """The reference's own engine unit tests, restated against an InversusEnv-shaped facade.
 
-Each function takes `make(width, height)` and follows one test of /root/reference/tests
+Each function takes `make(width, height)` and follows one test of the original project's tests/
 (file:line cited). Board extents are read back from the env (`env.width`) so the same bodies
 run on the oracle at the reference's board sizes and on the CUDA product's fixed 15x10 board.
 Height-1 boards of the reference tests are row 0 of whatever board the facade provides.

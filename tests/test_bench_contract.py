@@ -22,7 +22,7 @@ def _run(args, timeout=600):
 
 def test_reference_arm_line():
     d = _run(["--impl", "reference", "--steps", "4", "--warmup", "3", "--cpu-sample-envs", "2048"])
-    assert BASE_KEYS <= set(d) and d["impl"] == "reference"
+    assert BASE_KEYS <= set(d) and d["impl"] == "reference" and d["steps"] == 4
     assert d["metric"] == "env_steps_per_sec" and d["unit"] == "env-steps/s" and d["higher_is_better"] is True
     assert d["value"] > 0 and d["vs_baseline"] is None and d["data"] == "synthetic"
     staged = os.path.exists(os.path.join(ROOT, "oracle", "_ref", "inversus_rl", "env_wrappers.py"))
@@ -79,6 +79,37 @@ def test_b200_arm_line():
     assert d["config"]["preroll_steps"] == 500 + 100 - 3       # timed steps lie past the first episode timeout
     ev = d["e2e_variants"]["obs_stay_on_device_episode_events"]
     assert ev["value"] > 0 and ev["d2h_bytes_per_step"] < d["e2e_variants"]["obs_stay_on_device"]["d2h_bytes_per_step"]
+
+
+def test_reference_arm_refuses_dump_outputs(tmp_path):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "2",
+                        "--dump-outputs", str(tmp_path / "d")], capture_output=True, text=True, timeout=120, cwd=ROOT)
+    assert r.returncode != 0 and "--dump-outputs" in r.stderr and not os.path.exists(tmp_path / "d")
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_last_timed_step_and_reproducible(tmp_path):
+    """Two runs with the same arguments write identical files: float32/float64 arrays of the sampled
+    envs' outputs of the last timed step, P2's view included in selfplay."""
+    import numpy as np
+    dumps = []
+    for k in range(2):
+        out = tmp_path / str(k)
+        d = _run(["--mode", "selfplay", "--envs-per-gpu", "300000", "--steps", "5", "--warmup", "3", "--e2e-steps", "0",
+                  "--cpu-seconds", "0", "--ppo", "0", "--dump-outputs", str(out)])
+        assert d["steps"] == 5 and d["gpu_launches"] == 5
+        assert sum(os.path.getsize(out / f) for f in os.listdir(out)) <= 64 << 20
+        dumps.append({f[:-4]: np.load(out / f) for f in os.listdir(out)})
+    a, b = dumps
+    assert set(a) == {"env_index", "obs_env_index", "obs", "extra", "reward", "done", "info", "episode_steps",
+                      "episode_return", "obs_p2", "extra_p2"}
+    assert set(b) == set(a) and all(np.array_equal(a[k], b[k]) for k in a)
+    assert all(v.dtype in (np.float32, np.float64) for v in a.values())
+    rows = a["env_index"]
+    assert len(rows) == 1 << 18 and np.all(np.diff(rows) > 0) and rows[-1] < 300000
+    assert a["obs"].shape == a["obs_p2"].shape == (2048, 12, 10, 15) and np.isin(a["obs_env_index"], rows).all()
+    assert a["reward"].shape == a["done"].shape == (1 << 18,) and a["extra_p2"].shape == (1 << 18, 4)
+    assert set(np.unique(a["obs"])) <= {0.0, 1.0} and set(np.unique(a["done"])) <= {0.0, 1.0}
 
 
 @pytest.mark.gpu

@@ -101,13 +101,13 @@ def test_selfplay_training_runs(tmp_path):
     assert out["steps"] == 512 * 48 and np.isfinite(out["policy_loss"]) and np.isfinite(out["entropy"])
 
 
-def test_ppo_learns_to_beat_the_easy_dummy():
+def test_ppo_learns_to_beat_the_easy_dummy(tmp_path):
     """Learning-quality smoke: against the easy (sitting-duck) dummy a short run must raise the
     kill frequency (wins per 1000 env-steps in the last logging window) clearly above what the
     same untrained policy achieves (lr = 0 control, same seed)."""
     import torch
     from inversus_b200 import train_vs_dummy
-    kw = dict(num_envs=4096, log_dir="/tmp/inv_learn", opponent_difficulty="easy", precision="bf16",
+    kw = dict(num_envs=4096, log_dir=str(tmp_path), opponent_difficulty="easy", precision="bf16",
               rollout_steps=64, batch_size=8192, seed=5, quiet=True, save=False)
     torch.manual_seed(0)
     base = train_vs_dummy(total_steps=4096 * 64 * 2, lr=0.0, **kw)

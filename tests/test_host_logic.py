@@ -21,9 +21,9 @@ def test_discrete_to_action():  # tests/test_rl_env_wrapper.py:25 of the referen
 
 
 def test_action_table_agrees_with_the_live_reference():
-    from ref_harness import import_reference, reference_available
+    from ref_harness import SKIP_REASON, import_reference, reference_available
     if not reference_available():
-        pytest.skip("/root/reference not present")
+        pytest.skip(SKIP_REASON)
     ew = import_reference()
     from inversus_b200 import discrete_to_action
     for i in range(13):

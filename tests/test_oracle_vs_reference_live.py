@@ -1,5 +1,5 @@
-"""Checks against the LIVE Python reference. Builder-container only: skipped when
-/root/reference is absent (it is on the GPU box). Nothing here runs under -m gpu.
+"""Checks against the LIVE Python reference (tests/ref_harness.py): skipped unless
+INVERSUS_REFERENCE_ROOT names a checkout of the original project. Nothing here runs under -m gpu.
 
 1. The restated known-answer tests (tests/reference_kat.py) are first run against the real
    `inversus.core.InversusEnv`, proving the restatements are true of the reference itself.
@@ -10,11 +10,10 @@ import numpy as np
 import pytest
 
 import reference_kat as K
-from ref_harness import DrawShim, import_reference, reference_available
+from ref_harness import SKIP_REASON, DrawShim, import_reference, reference_available
 from engine_facade import Bullet, P1, P2
 
-pytestmark = [pytest.mark.live_reference,
-              pytest.mark.skipif(not reference_available(), reason="/root/reference not present")]
+pytestmark = [pytest.mark.live_reference, pytest.mark.skipif(not reference_available(), reason=SKIP_REASON)]
 
 
 class ReferenceEngine:

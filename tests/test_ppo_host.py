@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 import torch
 
-from ref_harness import reference_available
+from ref_harness import SKIP_REASON, reference_available
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
@@ -44,7 +44,7 @@ def test_per_env_gae_is_the_flat_gae_of_each_column():
         assert np.array_equal(adv[:, n], a1[:, 0]) and np.array_equal(ret[:, n], r1[:, 0])
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not present")
+@pytest.mark.skipif(not reference_available(), reason=SKIP_REASON)
 def test_policy_forward_is_bit_identical_to_the_live_reference():
     from ref_harness import import_reference
     import_reference()
@@ -62,7 +62,7 @@ def test_policy_forward_is_bit_identical_to_the_live_reference():
     assert (a[0] - c[0]).abs().max() < 2e-2 and (a[1] - c[1]).abs().max() < 2e-2
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not present")
+@pytest.mark.skipif(not reference_available(), reason=SKIP_REASON)
 def test_ppo_update_is_bit_identical_to_the_live_reference():
     """Same buffers, same numpy shuffle seed -> identical GAE, losses (1e-6) and parameters (exact)."""
     from ref_harness import import_reference
