@@ -347,66 +347,6 @@ cudaError_t launch(const Params &p, int dt, bool p2v, int sm_count, cudaStream_t
 #undef INV_CASE
 }
 
-// packed <-> canonical (host side; used by export/import only)
-void unpack_host(const uint32_t *pl[5], int64_t i, inv_env_state *o)
-{
-    const uint32_t *a = pl[0] + 4 * i, *b = pl[1] + 4 * i, *c = pl[2] + 4 * i, *d = pl[3] + 4 * i, *e = pl[4] + 4 * i;
-    memset(o, 0, sizeof(*o));
-    o->tiles[0] = a[0]; o->tiles[1] = a[1]; o->tiles[2] = a[2]; o->tiles[3] = a[3]; o->tiles[4] = b[0];
-    const uint32_t pw[2] = {b[1], b[2]};
-    int32_t *pp[2] = {o->p1, o->p2};
-    for (int k = 0; k < 2; ++k) {
-        pp[k][0] = pw[k] & 15; pp[k][1] = (pw[k] >> 4) & 15; pp[k][2] = (pw[k] >> 8) & 7;
-        pp[k][3] = (pw[k] >> 11) & 31; pp[k][4] = (pw[k] >> 16) & 1;
-    }
-    o->n_bullets = (b[1] >> 20) & 31;
-    o->step_count = (int32_t)b[3];
-    o->episode = c[0];
-    uint64_t bits = (uint64_t)c[1] | ((uint64_t)c[2] << 32);
-    memcpy(&o->episode_return, &bits, 8);
-    const uint32_t w[8] = {d[0], d[1], d[2], d[3], e[0], e[1], e[2], e[3]};
-    for (int s = 0; s < o->n_bullets && s < INV_MAX_BULLETS; ++s) {
-        const uint32_t bl = (w[s >> 1] >> ((s & 1) * 16)) & 0xFFFFu;
-        o->bullets[s][0] = (int8_t)(bl & 15); o->bullets[s][1] = (int8_t)((bl >> 4) & 15);
-        o->bullets[s][2] = (int8_t)((bl >> 8) & 3); o->bullets[s][3] = (int8_t)((bl >> 10) & 1);
-    }
-}
-
-bool pack_host(const inv_env_state *in, uint32_t *pl[5], int64_t i)
-{
-    uint32_t *a = pl[0] + 4 * i, *b = pl[1] + 4 * i, *c = pl[2] + 4 * i, *d = pl[3] + 4 * i, *e = pl[4] + 4 * i;
-    if (in->tiles[4] >> 22) return false;
-    if (in->n_bullets < 0 || in->n_bullets > INV_MAX_BULLETS) return false;
-    a[0] = in->tiles[0]; a[1] = in->tiles[1]; a[2] = in->tiles[2]; a[3] = in->tiles[3]; b[0] = in->tiles[4];
-    const int32_t *pp[2] = {in->p1, in->p2};
-    uint32_t pw[2];
-    for (int k = 0; k < 2; ++k) {
-        const int32_t *q = pp[k];
-        if (q[0] < 0 || q[0] >= INV_BOARD_W || q[1] < 0 || q[1] >= INV_BOARD_H || q[2] < 0 || q[2] > 7 ||
-            q[3] < 0 || q[3] > 31 || (q[4] != 0 && q[4] != 1))
-            return false;
-        pw[k] = (uint32_t)q[0] | ((uint32_t)q[1] << 4) | ((uint32_t)q[2] << 8) | ((uint32_t)q[3] << 11) | ((uint32_t)q[4] << 16);
-    }
-    b[1] = pw[0] | ((uint32_t)in->n_bullets << 20);
-    b[2] = pw[1];
-    b[3] = (uint32_t)in->step_count;
-    c[0] = in->episode;
-    uint64_t bits;
-    memcpy(&bits, &in->episode_return, 8);
-    c[1] = (uint32_t)bits; c[2] = (uint32_t)(bits >> 32); c[3] = 0;
-    uint32_t w[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    for (int s = 0; s < in->n_bullets; ++s) {
-        const int8_t *q = in->bullets[s];
-        if (q[0] < 0 || q[0] >= INV_BOARD_W || q[1] < 0 || q[1] >= INV_BOARD_H || q[2] < 0 || q[2] > 3 || q[3] < 0 || q[3] > 1)
-            return false;
-        const uint32_t bl = (uint32_t)q[0] | ((uint32_t)q[1] << 4) | ((uint32_t)q[2] << 8) | ((uint32_t)q[3] << 10);
-        w[s >> 1] |= bl << ((s & 1) * 16);
-    }
-    d[0] = w[0]; d[1] = w[1]; d[2] = w[2]; d[3] = w[3];
-    e[0] = w[4]; e[1] = w[5]; e[2] = w[6]; e[3] = w[7];
-    return true;
-}
-
 } // namespace
 
 extern "C" {
@@ -1092,15 +1032,16 @@ int inv_export_state(inv_sim *s, inv_env_state *out, int64_t first, int64_t coun
     if (count == 0) return INV_OK;
     DeviceGuard g(s->cfg.device);
     CUDA_TRY(cudaDeviceSynchronize());
-    std::vector<uint32_t> buf((size_t)count * 20);
-    const uint32_t *pl[5];
-    for (int k = 0; k < 5; ++k) {
-        uint32_t *dst = buf.data() + (size_t)k * count * 4;
-        CUDA_TRY(cudaMemcpy(dst, reinterpret_cast<const char *>(s->state) + ((size_t)k * s->n + first) * 16,
-                            (size_t)count * 16, cudaMemcpyDeviceToHost));
-        pl[k] = dst;
+    std::vector<uint4> buf((size_t)count * 5); // [5][count]: a plane set with stride count
+    for (int k = 0; k < 5; ++k)
+        CUDA_TRY(cudaMemcpy(buf.data() + (size_t)k * count, s->state + (size_t)k * s->n + first, (size_t)count * 16,
+                            cudaMemcpyDeviceToHost));
+    for (int64_t i = 0; i < count; ++i) {
+        Env e;
+        uint16_t sb[kSlots];
+        load_env<1>(e, sb, buf.data(), count, i);
+        env_to_canonical(e, sb, out[i]);
     }
-    for (int64_t i = 0; i < count; ++i) unpack_host(pl, i, &out[i]);
     return INV_OK;
 }
 
@@ -1110,15 +1051,17 @@ int inv_import_state(inv_sim *s, const inv_env_state *in, int64_t first, int64_t
     if (first < 0 || count < 0 || first + count > s->n) return fail(INV_ERR_INVALID_ARG, "inv_import_state: bad range");
     if (count == 0) return INV_OK;
     DeviceGuard g(s->cfg.device);
-    std::vector<uint32_t> buf((size_t)count * 20);
-    uint32_t *pl[5];
-    for (int k = 0; k < 5; ++k) pl[k] = buf.data() + (size_t)k * count * 4;
-    for (int64_t i = 0; i < count; ++i)
-        if (!pack_host(&in[i], pl, i)) return fail(INV_ERR_INVALID_ARG, "inv_import_state: field out of range");
+    std::vector<uint4> buf((size_t)count * 5); // [5][count]: a plane set with stride count
+    for (int64_t i = 0; i < count; ++i) {
+        Env e;
+        uint16_t sb[kSlots];
+        if (!env_from_canonical(in[i], e, sb)) return fail(INV_ERR_INVALID_ARG, "inv_import_state: field out of range");
+        store_env<1>(e, sb, buf.data(), count, i);
+    }
     CUDA_TRY(cudaDeviceSynchronize());
     for (int k = 0; k < 5; ++k)
-        CUDA_TRY(cudaMemcpy(reinterpret_cast<char *>(s->state) + ((size_t)k * s->n + first) * 16, pl[k],
-                            (size_t)count * 16, cudaMemcpyHostToDevice));
+        CUDA_TRY(cudaMemcpy(s->state + (size_t)k * s->n + first, buf.data() + (size_t)k * count, (size_t)count * 16,
+                            cudaMemcpyHostToDevice));
     s->was_reset = true;
     return INV_OK;
 }

@@ -28,8 +28,13 @@
 #include <cuda_runtime.h>
 #endif
 #include <stdint.h>
+#include <string.h>
 
 #include "../../include/inversus_b200.h"
+
+// The packed-state codec (Env, pack_*/unpack_*, load_env, store_env) is shared by the kernels and
+// the host side of inv_export_state / inv_import_state.
+#define INV_HD __host__ __device__ __forceinline__
 
 namespace inv {
 
@@ -143,25 +148,62 @@ struct Env {
     double ret;
 };
 
-__device__ __forceinline__ uint32_t pack_player(const Env &s, int i)
+INV_HD uint32_t pack_player(const Env &s, int i)
 {
     return (uint32_t)s.x[i] | ((uint32_t)s.y[i] << 4) | ((uint32_t)s.ammo[i] << 8) |
            ((uint32_t)s.reload[i] << 11) | ((uint32_t)s.alive[i] << 16);
 }
-__device__ __forceinline__ void unpack_player(Env &s, int i, uint32_t w)
+INV_HD void unpack_player(Env &s, int i, uint32_t w)
 {
     s.x[i] = w & 15; s.y[i] = (w >> 4) & 15; s.ammo[i] = (w >> 8) & 7;
     s.reload[i] = (w >> 11) & 31; s.alive[i] = (w >> 16) & 1;
 }
 
 // bullets live in a private shared-memory column: sb[slot * E]; 16-bit x | y<<4 | dir<<8 | owner<<10
-__device__ __forceinline__ uint32_t pack_bullet(int x, int y, int dir, int owner)
+INV_HD uint32_t pack_bullet(int x, int y, int dir, int owner)
 {
     return (uint32_t)x | ((uint32_t)y << 4) | ((uint32_t)dir << 8) | ((uint32_t)owner << 10);
 }
+INV_HD void unpack_bullet(uint32_t b, int8_t (&q)[4]) // x, y, dir, owner
+{
+    q[0] = (int8_t)(b & 15); q[1] = (int8_t)((b >> 4) & 15); q[2] = (int8_t)((b >> 8) & 3); q[3] = (int8_t)((b >> 10) & 1);
+}
+
+// the episode return is stored as its two 32-bit halves
+INV_HD double double_from_words(uint32_t lo, uint32_t hi)
+{
+#ifdef __CUDA_ARCH__
+    return __hiloint2double((int)hi, (int)lo);
+#else
+    const uint64_t bits = ((uint64_t)hi << 32) | lo;
+    double d;
+    memcpy(&d, &bits, 8);
+    return d;
+#endif
+}
+INV_HD uint32_t double_lo_word(double d)
+{
+#ifdef __CUDA_ARCH__
+    return (uint32_t)__double2loint(d);
+#else
+    uint64_t bits;
+    memcpy(&bits, &d, 8);
+    return (uint32_t)bits;
+#endif
+}
+INV_HD uint32_t double_hi_word(double d)
+{
+#ifdef __CUDA_ARCH__
+    return (uint32_t)__double2hiint(d);
+#else
+    uint64_t bits;
+    memcpy(&bits, &d, 8);
+    return (uint32_t)(bits >> 32);
+#endif
+}
 
 template <int E>
-__device__ __forceinline__ void load_env(Env &s, uint16_t *sb, const uint4 *st, int64_t stride, int64_t i)
+INV_HD void load_env(Env &s, uint16_t *sb, const uint4 *st, int64_t stride, int64_t i)
 {
     const uint4 a = st[i], b = st[stride + i], c = st[2 * stride + i];
     const uint4 d = st[3 * stride + i], e = st[4 * stride + i];
@@ -171,7 +213,7 @@ __device__ __forceinline__ void load_env(Env &s, uint16_t *sb, const uint4 *st, 
     unpack_player(s, 1, b.z);
     s.step = b.w;
     s.episode = c.x;
-    s.ret = __hiloint2double((int)c.z, (int)c.y);
+    s.ret = double_from_words(c.y, c.z);
     const uint32_t w[8] = {d.x, d.y, d.z, d.w, e.x, e.y, e.z, e.w};
 #pragma unroll
     for (int k = 0; k < 8; ++k) {
@@ -183,11 +225,11 @@ __device__ __forceinline__ void load_env(Env &s, uint16_t *sb, const uint4 *st, 
 }
 
 template <int E>
-__device__ __forceinline__ void store_env(const Env &s, const uint16_t *sb, uint4 *st, int64_t stride, int64_t i)
+INV_HD void store_env(const Env &s, const uint16_t *sb, uint4 *st, int64_t stride, int64_t i)
 {
     st[i] = make_uint4(s.t[0], s.t[1], s.t[2], s.t[3]);
     st[stride + i] = make_uint4(s.t[4], pack_player(s, 0) | ((uint32_t)s.nb << 20), pack_player(s, 1), s.step);
-    st[2 * stride + i] = make_uint4(s.episode, (uint32_t)__double2loint(s.ret), (uint32_t)__double2hiint(s.ret), 0u);
+    st[2 * stride + i] = make_uint4(s.episode, double_lo_word(s.ret), double_hi_word(s.ret), 0u);
     uint32_t w[8];
 #pragma unroll
     for (int k = 0; k < 8; ++k) {
@@ -197,6 +239,49 @@ __device__ __forceinline__ void store_env(const Env &s, const uint16_t *sb, uint
     }
     st[3 * stride + i] = make_uint4(w[0], w[1], w[2], w[3]);
     st[4 * stride + i] = make_uint4(w[4], w[5], w[6], w[7]);
+}
+
+// Env + its bullet column (E = 1) <-> the canonical inv_env_state of the C ABI (host only).
+inline void env_to_canonical(const Env &s, const uint16_t *sb, inv_env_state &o)
+{
+    o = inv_env_state{};
+    int32_t *pp[2] = {o.p1, o.p2};
+    for (int k = 0; k < 5; ++k) o.tiles[k] = s.t[k];
+    for (int i = 0; i < 2; ++i) {
+        pp[i][0] = s.x[i]; pp[i][1] = s.y[i]; pp[i][2] = s.ammo[i]; pp[i][3] = s.reload[i]; pp[i][4] = s.alive[i];
+    }
+    o.n_bullets = s.nb;
+    for (int k = 0; k < s.nb && k < kSlots; ++k) unpack_bullet(sb[k], o.bullets[k]);
+    o.step_count = (int32_t)s.step;
+    o.episode = s.episode;
+    o.episode_return = s.ret;
+}
+
+// false if a field does not fit the packed layout (or the board)
+inline bool env_from_canonical(const inv_env_state &in, Env &s, uint16_t *sb)
+{
+    if (in.tiles[4] >> (kTiles - 128)) return false; // bits beyond the 150 tiles
+    if (in.n_bullets < 0 || in.n_bullets > kSlots) return false;
+    const int32_t *pp[2] = {in.p1, in.p2};
+    for (int k = 0; k < 5; ++k) s.t[k] = in.tiles[k];
+    for (int i = 0; i < 2; ++i) {
+        const int32_t *q = pp[i];
+        if (q[0] < 0 || q[0] >= kW || q[1] < 0 || q[1] >= kH || q[2] < 0 || q[2] > 7 || q[3] < 0 || q[3] > 31 ||
+            (q[4] != 0 && q[4] != 1))
+            return false;
+        s.x[i] = q[0]; s.y[i] = q[1]; s.ammo[i] = q[2]; s.reload[i] = q[3]; s.alive[i] = q[4];
+    }
+    s.nb = in.n_bullets;
+    for (int k = 0; k < s.nb; ++k) {
+        const int8_t *q = in.bullets[k];
+        if (q[0] < 0 || q[0] >= kW || q[1] < 0 || q[1] >= kH || q[2] < 0 || q[2] > 3 || q[3] < 0 || q[3] > 1)
+            return false;
+        sb[k] = (uint16_t)pack_bullet(q[0], q[1], q[2], q[3]);
+    }
+    s.step = (uint32_t)in.step_count;
+    s.episode = in.episode;
+    s.ret = in.episode_return;
+    return true;
 }
 
 // ---- tile bit access on the 5 register words (select chains: no local memory, no smem) ----
@@ -586,6 +671,42 @@ __device__ __forceinline__ StepResult rl_step(Env &s, uint16_t *sb, int a1, int 
     return o;
 }
 
+// One engine method of core.py, selected by p.phase (inv_debug_phase); returns the method's result.
+template <int E>
+__device__ __forceinline__ uint8_t debug_phase(Env &s, uint16_t *sb, const Params &p, uint32_t gid, const uint32_t *trow)
+{
+    int res = 0;
+    switch (p.phase) {
+    case INV_PHASE_TRY_MOVE:
+        res = p.pid ? try_move(s, 1, p.arg) : try_move(s, 0, p.arg);
+        break;
+    case INV_PHASE_SPAWN_BULLET:
+        res = p.pid ? spawn_bullet<E>(s, sb, 1, p.arg, p.status) : spawn_bullet<E>(s, sb, 0, p.arg, p.status);
+        break;
+    case INV_PHASE_WIDE_SHOT:
+        res = p.pid ? spawn_wide_shot<E>(s, sb, 1, p.arg, p.status) : spawn_wide_shot<E>(s, sb, 0, p.arg, p.status);
+        break;
+    case INV_PHASE_RELOAD: reload_ammo(s); break;
+    case INV_PHASE_UPDATE_BULLETS: update_bullets<E>(s, sb); break;
+    case INV_PHASE_STEP_PLAYERS: step_players<E>(s, sb, p.arg, p.arg2, p.status); break;
+    case INV_PHASE_ENGINE_RESET: {
+        s.episode += 1u;
+        Draws dr;
+        dr.init(p, gid, s.episode, INV_STREAM_RESET, trow ? trow + INV_TABLE_RESET_OFF : nullptr);
+        engine_reset(s, dr);
+        break;
+    }
+    case INV_PHASE_DUMMY_POLICY: {
+        Draws dr;
+        dr.init(p, gid, s.episode, s.step, trow);
+        res = dummy_policy(s, dr, p.difficulty);
+        break;
+    }
+    default: break;
+    }
+    return (uint8_t)res;
+}
+
 #ifndef INV_HOST_BUILD
 // ---- observation formats: how many store chunks per env and how a chunk is expanded ----
 template <int DT> struct ObsFmt;
@@ -721,36 +842,7 @@ __global__ void __launch_bounds__(T) inv_kernel(const Params p)
             } else if (OP == OP_RESET) { // env_wrappers.py:272-284
                 rl_reset(s, p, gid, trow);
             } else if (OP == OP_DEBUG) {
-                int res = 0;
-                switch (p.phase) {
-                case INV_PHASE_TRY_MOVE:
-                    res = p.pid ? try_move(s, 1, p.arg) : try_move(s, 0, p.arg);
-                    break;
-                case INV_PHASE_SPAWN_BULLET:
-                    res = p.pid ? spawn_bullet<E>(s, sb, 1, p.arg, p.status) : spawn_bullet<E>(s, sb, 0, p.arg, p.status);
-                    break;
-                case INV_PHASE_WIDE_SHOT:
-                    res = p.pid ? spawn_wide_shot<E>(s, sb, 1, p.arg, p.status) : spawn_wide_shot<E>(s, sb, 0, p.arg, p.status);
-                    break;
-                case INV_PHASE_RELOAD: reload_ammo(s); break;
-                case INV_PHASE_UPDATE_BULLETS: update_bullets<E>(s, sb); break;
-                case INV_PHASE_STEP_PLAYERS: step_players<E>(s, sb, p.arg, p.arg2, p.status); break;
-                case INV_PHASE_ENGINE_RESET: {
-                    s.episode += 1u;
-                    Draws dr;
-                    dr.init(p, gid, s.episode, INV_STREAM_RESET, trow ? trow + INV_TABLE_RESET_OFF : nullptr);
-                    engine_reset(s, dr);
-                    break;
-                }
-                case INV_PHASE_DUMMY_POLICY: {
-                    Draws dr;
-                    dr.init(p, gid, s.episode, s.step, trow);
-                    res = dummy_policy(s, dr, p.difficulty);
-                    break;
-                }
-                default: break;
-                }
-                p.dbg[ei] = (uint8_t)res;
+                p.dbg[ei] = debug_phase<E>(s, sb, p, gid, trow);
             }
 
             if (OP != OP_OBS) store_env<E>(s, sb, p.state, p.stride, ei);

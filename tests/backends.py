@@ -5,6 +5,8 @@ import ctypes as C
 
 import numpy as np
 
+from oracle.oracle import STATE_DTYPE
+
 
 class OracleBackend:
     """The C oracle (oracle/inversus_oracle.c) as a scenario backend. Checker only."""
@@ -122,7 +124,6 @@ class PyLoopBackend:
             self.r.envs[int(i)].reset(None if table is None else table[int(i)])
 
     def state(self):
-        from oracle.oracle import STATE_DTYPE
         T = self.pl.Tile
         out = np.zeros(self.r.n, STATE_DTYPE)
         for i, e in enumerate(self.r.envs):
@@ -148,8 +149,8 @@ class PyLoopBackend:
 
 class HostKernelBackend:
     """The PRODUCT's own step logic (csrc/inversus_kernels.cuh: load_env, rl_step, rl_reset,
-    build_row, store_env) compiled for the host through tests/host_kernel/host_shim.h and driven
-    over the same packed-state planes the GPU uses. Test harness only: it lets the CPU suite replay
+    build_row, store_env) and canonical-state conversions compiled for the host through
+    tests/host_kernel/host_shim.h and driven over the same packed-state planes the GPU uses. Test harness only: it lets the CPU suite replay
     the golden fixtures through the real kernel logic without a GPU."""
 
     _lib = None
@@ -178,7 +179,9 @@ class HostKernelBackend:
         self.selfplay = sc["mode"] == "selfplay"
         n = self.n
         self.planes = np.zeros((5, n, 4), np.uint32)
-        self.planes[2, :, 0] = 0xFFFFFFFF  # "no episode yet", like inv_create
+        st = np.zeros(n, STATE_DTYPE)
+        st["episode"] = 0xFFFFFFFF  # "no episode yet", like inv_create
+        self.import_state(st)
         self.obs1 = np.zeros((n, 12, 10, 15), np.float32)
         self.obs2 = np.zeros((n, 12, 10, 15), np.float32)
         self.extra1 = np.zeros((n, 4), np.float32)
@@ -220,26 +223,51 @@ class HostKernelBackend:
             out["obs2"], out["extra2"] = self.obs2, self.extra2
         return out
 
-    def state(self):
-        """Unpack the planes (DESIGN.md section 3) into the canonical state array."""
-        from oracle.oracle import STATE_DTYPE
-        pl, n = self.planes, self.n
-        out = np.zeros(n, STATE_DTYPE)
-        out["tiles"][:, :4] = pl[0]
-        out["tiles"][:, 4] = pl[1, :, 0]
-        for name, w in (("p1", pl[1, :, 1]), ("p2", pl[1, :, 2])):
-            out[name] = np.stack([w & 15, (w >> 4) & 15, (w >> 8) & 7, (w >> 11) & 31, (w >> 16) & 1], axis=1)
-        nb = (pl[1, :, 1] >> 20) & 31
-        out["n_bullets"] = nb
-        out["step_count"] = pl[1, :, 3].astype(np.int32)
-        out["episode"] = pl[2, :, 0]
-        out["episode_return"] = (pl[2, :, 1].astype(np.uint64) | (pl[2, :, 2].astype(np.uint64) << np.uint64(32))).view(np.float64)
-        words = np.concatenate([pl[3], pl[4]], axis=1)  # [n, 8]
-        for s in range(16):
-            b = (words[:, s >> 1] >> ((s & 1) * 16)) & 0xFFFF
-            live = s < nb
-            out["bullets"][:, s] = np.where(live[:, None], np.stack([b & 15, (b >> 4) & 15, (b >> 8) & 3, (b >> 10) & 1], 1), 0)
+    def export_state(self, first=0, count=None):
+        """Canonical state of envs [first, first+count), decoded by the product's own conversion."""
+        count = self.n - first if count is None else count
+        out = np.zeros(count, STATE_DTYPE)
+        self.lib().hk_export_state(self._p(self.planes), C.c_int64(self.n), C.c_int64(first), C.c_int64(count),
+                                   self._p(out))
         return out
+
+    def import_state(self, state, first=0):
+        st = np.ascontiguousarray(state, STATE_DTYPE)
+        if self.lib().hk_import_state(self._p(self.planes), C.c_int64(self.n), C.c_int64(first),
+                                      C.c_int64(len(st)), self._p(st)) != 0:
+            raise ValueError("hk_import_state: field out of range")
+
+    def state(self):
+        return self.export_state()
 
     def obs(self):
         return self.obs1, self.extra1, self.obs2, self.extra2
+
+
+def check_state_import_export(export, import_):
+    """Canonical state through a product's import/export: a round trip at an offset is exact, and
+    every field outside the packed layout or the board is rejected. export(first=0, count=None) and
+    import_(state, first=0) act on at least 11 envs after a reset."""
+    import pytest
+    st = export()
+    st["bullets"][3, :2] = [[4, 5, 1, 0], [9, 2, 3, 1]]
+    st["n_bullets"][3] = 2
+    st["episode_return"][3] = -1.2345678901234567
+    st["p1"][3] = (14, 9, 0, 29, 0)
+    import_(st[3:4], first=10)
+    back = export(10, 1)
+    for f in st.dtype.names:
+        assert np.array_equal(back[f][0], st[f][3]), f
+    for field, bad in (("p1", (15, 0, 0, 0, 1)), ("p2", (0, 10, 0, 0, 1)), ("p1", (0, 0, 8, 0, 1)), ("p1", (0, 0, 0, 0, 2))):
+        x = st[:1].copy()
+        x[field][0] = bad
+        with pytest.raises(ValueError):
+            import_(x)
+    x = st[:1].copy()
+    x["n_bullets"][0] = 17
+    with pytest.raises(ValueError):
+        import_(x)
+    x = st[:1].copy()
+    x["tiles"][0][4] = 1 << 22  # bit beyond the 150 tiles
+    with pytest.raises(ValueError):
+        import_(x)

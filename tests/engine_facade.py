@@ -2,13 +2,16 @@
 
 `OracleEngine` drives oracle/inversus_oracle.c one engine call at a time (core.py method names);
 `CudaEngine` (tests/test_cuda_reference_kat.py) drives the CUDA product through its debug-phase
-entry point with the same surface. Directions/ids use the product's integer encoding:
+entry point with the same surface, and `HostKernelEngine` (tests/test_host_kernel.py) the same
+engine functions compiled for the host. Directions/ids use the product's integer encoding:
 UP, RIGHT, DOWN, LEFT = 0..3; P1, P2 = 0, 1; BLACK, WHITE = 0, 1.
 """
 from __future__ import annotations
 
 import ctypes as C
 from collections import namedtuple
+
+import numpy as np
 
 Bullet = namedtuple("Bullet", "x y dir owner")
 UP, RIGHT, DOWN, LEFT = 0, 1, 2, 3
@@ -147,41 +150,38 @@ class OracleEngine:
         return {0: None, 1: P1, 2: P2}[self.L.orc_get_winner(C.byref(self.e))]
 
     def observation(self, viewer=P1):
-        import numpy as np
         g = np.zeros((12, self.height, self.width), np.float32)
         x = np.zeros(4, np.float32)
         self.L.orc_build_obs(C.byref(self.e), viewer, g.ctypes.data, x.ctypes.data)
         return g, x
 
 
-class CudaEngine:
-    """The CUDA product behind core.py's method names: each call runs ONE engine method on the
-    device through inv_debug_phase (the same __device__ functions the fused step kernel inlines).
-    Fixed 15x10 board; field pokes go through inv_export_state / inv_import_state."""
+class _StateEngine:
+    """core.py's method names over one env of the product: field pokes edit the canonical state
+    (STATE_DTYPE) and go through the product's import/export; each engine call runs ONE engine
+    method through the debug-phase dispatch the fused step kernel is built from. Fixed 15x10 board.
+    Subclasses provide _export, _import, _run_phase and _observation."""
 
-    def __init__(self, width=15, height=10, seed=1234):
-        from inversus_b200 import BatchedInversus, _capi
+    def __init__(self, width, height):
+        from inversus_b200 import _capi
         assert width <= 15 and height <= 10
         self.capi = _capi
-        self.sim = BatchedInversus(1, "selfplay", "hard", 500, seed=seed, auto_reset=False)
         self.width, self.height = 15, 10
         self.player_color = BLACK
-        self.sim.reset()
         self._pull()
 
     def _pull(self):
-        self._st = self.sim.export_state()
+        self._st = self._export()
         self._dirty = False
 
     def _push(self):
         if self._dirty:
-            self.sim.import_state(self._st)
+            self._import(self._st)
             self._dirty = False
 
     def _call(self, phase, pid=0, arg=0, arg2=0):
         self._push()
-        res = int(self.sim.debug_phase(phase, pid, arg, arg2).cpu()[0])
-        assert self.sim.poll_status() == 0
+        res = self._run_phase(phase, pid, arg, arg2)
         self._pull()
         return res
 
@@ -289,149 +289,60 @@ class CudaEngine:
 
     def observation(self, viewer=P1):
         self._push()
+        return self._observation(viewer)
+
+
+class CudaEngine(_StateEngine):
+    """The CUDA product: inv_debug_phase on the device, inv_export_state / inv_import_state."""
+
+    def __init__(self, width=15, height=10, seed=1234):
+        from inversus_b200 import BatchedInversus
+        self.sim = BatchedInversus(1, "selfplay", "hard", 500, seed=seed, auto_reset=False)
+        self.sim.reset()
+        super().__init__(width, height)
+
+    def _export(self):
+        return self.sim.export_state()
+
+    def _import(self, st):
+        self.sim.import_state(st)
+
+    def _run_phase(self, phase, pid, arg, arg2):
+        res = int(self.sim.debug_phase(phase, pid, arg, arg2).cpu()[0])
+        assert self.sim.poll_status() == 0
+        return res
+
+    def _observation(self, viewer):
         g, e = self.sim.obs_from_packed(self.sim.snapshot(), view=viewer, obs_dtype="f32")
         return g[0].cpu().numpy(), e[0].cpu().numpy()
 
 
-class HostKernelEngine:
-    """The product's engine functions compiled for the host (tests/host_kernel) behind core.py's
-    method names: the CPU-side twin of CudaEngine, same device functions, no GPU needed."""
+class HostKernelEngine(_StateEngine):
+    """The product's engine functions and state conversions compiled for the host (tests/host_kernel):
+    the CPU-side twin of CudaEngine, no GPU needed."""
 
     def __init__(self, width=15, height=10, seed=1234):
-        import ctypes as C_
-        import numpy as np
         from backends import HostKernelBackend
-        assert width <= 15 and height <= 10
-        self.C, self.np = C_, np
-        self.lib = HostKernelBackend.lib()
         self.b = HostKernelBackend(dict(n=1, mode="selfplay", difficulty="hard", max_steps=500, seed=seed))
-        self.width, self.height = 15, 10
-        self.player_color = BLACK
         self.b.reset(None)
+        super().__init__(width, height)
 
-    # packed-plane accessors (DESIGN.md section 3)
-    def _pw(self, i):
-        return int(self.b.planes[1, 0, 1 + i])
+    def _export(self):
+        return self.b.export_state()
 
-    def _set_pw(self, i, w):
-        self.b.planes[1, 0, 1 + i] = w
+    def _import(self, st):
+        self.b.import_state(st)
 
-    def _pv(self, i):
-        fields = {"x": (0, 15), "y": (4, 15), "ammo": (8, 7), "reload_counter": (11, 31), "alive": (16, 1)}
-
-        def get(k):
-            sh, m = fields[k]
-            return (self._pw(i) >> sh) & m
-
-        def set_(k, v):
-            sh, m = fields[k]
-            self._set_pw(i, (self._pw(i) & ~(m << sh)) | ((int(v) & m) << sh))
-        return _PlayerView(get, set_)
-
-    @property
-    def player1(self):
-        return self._pv(0)
-
-    @property
-    def player2(self):
-        return self._pv(1)
-
-    player_x = property(lambda s: s.player1.x, lambda s, v: setattr(s.player1, "x", v))
-
-    @property
-    def player_y(self):
-        return self.player1.y
-
-    @player_y.setter
-    def player_y(self, v):
-        self.player1.y = v
-        self.bullets = []  # core.py:180-181
-
-    @property
-    def bullets(self):
-        n = (self._pw(0) >> 20) & 31
-        words = [int(w) for w in list(self.b.planes[3, 0]) + list(self.b.planes[4, 0])]
-        out = []
-        for s in range(n):
-            b = (words[s >> 1] >> ((s & 1) * 16)) & 0xFFFF
-            out.append(Bullet(b & 15, (b >> 4) & 15, (b >> 8) & 3, (b >> 10) & 1))
-        return out
-
-    @bullets.setter
-    def bullets(self, lst):
-        words = [0] * 8
-        for s, b in enumerate(lst):
-            words[s >> 1] |= (b.x | (b.y << 4) | (b.dir << 8) | (b.owner << 10)) << ((s & 1) * 16)
-        self.b.planes[3, 0] = words[:4]
-        self.b.planes[4, 0] = words[4:]
-        self._set_pw(0, (self._pw(0) & ~(31 << 20)) | (len(lst) << 20))
-
-    def get_bullets(self):
-        return self.bullets
-
-    def _tile_word(self, i):
-        return (0, i >> 5) if (i >> 5) < 4 else (1, 0)
-
-    def _get_tile(self, x, y):
-        if not (0 <= x < self.width and 0 <= y < self.height):
-            raise IndexError
-        i = y * 15 + x
-        pl, w = self._tile_word(i)
-        return (int(self.b.planes[pl, 0, w]) >> (i & 31)) & 1
-
-    def _set_tile(self, x, y, c):
-        if not (0 <= x < self.width and 0 <= y < self.height):
-            raise IndexError
-        i = y * 15 + x
-        pl, w = self._tile_word(i)
-        v = int(self.b.planes[pl, 0, w])
-        self.b.planes[pl, 0, w] = (v | (1 << (i & 31))) if c else (v & ~(1 << (i & 31)))
-
-    def _call(self, phase, pid=0, arg=0, arg2=0):
-        C_, np = self.C, self.np
+    def _run_phase(self, phase, pid, arg, arg2):
+        b = self.b
         res = np.zeros(1, np.uint8)
-        rc = self.lib.hk_debug(self.b.planes.ctypes.data_as(C_.c_void_p), C_.c_int64(1), phase, pid, arg, arg2, 1,
-                               C_.c_uint64(self.b.seed), C_.c_uint32(0), res.ctypes.data_as(C_.c_void_p),
-                               self.b.status.ctypes.data_as(C_.c_void_p))
-        assert rc == 0 and self.b.status[0] == 0
+        rc = b.lib().hk_debug(b._p(b.planes), C.c_int64(1), phase, pid, arg, arg2, 1, C.c_uint64(b.seed), C.c_uint32(0),
+                              b._p(res), b._p(b.status))
+        assert rc == 0 and b.status[0] == 0
         return int(res[0])
 
-    def reset(self):
-        self._call(6)
-
-    def try_move_player(self, d, pid=P1):
-        return bool(self._call(0, pid, d))
-
-    def spawn_bullet(self, d, pid=P1):
-        return bool(self._call(1, pid, d))
-
-    def spawn_wide_shot(self, pid, d):
-        return bool(self._call(2, pid, d))
-
-    def _reload_ammo(self):
-        self._call(3)
-
-    def update_bullets(self):
-        self._call(4)
-
-    def step_players(self, a1, a2):
-        self._call(5, 0, a1, a2)
-
-    def step(self, a1):
-        self.step_players(a1, NONE)
-
-    def is_round_over(self):
-        return not (self.player1.alive and self.player2.alive)
-
-    def get_winner(self):
-        a1, a2 = self.player1.alive, self.player2.alive
-        if a1 and a2:
-            return None
-        return P2 if (a2 and not a1) else (P1 if (a1 and not a2) else None)
-
-    def observation(self, viewer=P1):
-        C_, np = self.C, self.np
+    def _observation(self, viewer):
+        b = self.b
         g, e = np.zeros((12, 10, 15), np.float32), np.zeros(4, np.float32)
-        self.lib.hk_observation(self.b.planes.ctypes.data_as(C_.c_void_p), C_.c_int64(1), C_.c_int64(0), viewer,
-                                g.ctypes.data_as(C_.c_void_p), e.ctypes.data_as(C_.c_void_p))
+        b.lib().hk_observation(b._p(b.planes), C.c_int64(1), C.c_int64(0), viewer, b._p(g), b._p(e))
         return g, e

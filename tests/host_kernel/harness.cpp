@@ -1,7 +1,8 @@
 // harness.cpp -- TEST INFRASTRUCTURE. Drives the product's own device functions (load_env,
-// rl_step, rl_reset, build_row, extra_vec, store_env of csrc/inversus_kernels.cuh), compiled for
-// the host through host_shim.h, over the same packed-state planes the GPU uses. One "thread" per
-// env, tile size E = 1. See tests/test_host_kernel.py.
+// rl_step, rl_reset, debug_phase, build_row, extra_vec, store_env of csrc/inversus_kernels.cuh) and
+// its canonical-state conversions, compiled for the host through host_shim.h, over the same
+// packed-state planes the GPU uses. One "thread" per env, tile size E = 1. See
+// tests/test_host_kernel.py.
 #define INV_HOST_BUILD 1
 #include "../../inversus-reinforcement-learning_b200/csrc/inversus_kernels.cuh"
 
@@ -85,37 +86,42 @@ int hk_step(uint32_t *planes, int64_t n, const int8_t *a1, const int8_t *a2, con
 int hk_debug(uint32_t *planes, int64_t n, int phase, int pid, int arg, int arg2, int difficulty, uint64_t seed,
              uint32_t env_id_base, uint8_t *result, uint32_t *status)
 {
+    if (phase < 0 || phase > INV_PHASE_DUMMY_POLICY) return -1;
     uint4 *st = reinterpret_cast<uint4 *>(planes);
     Params p = make_params(1, difficulty, 500, 0, seed, env_id_base, nullptr, status);
+    p.phase = phase; p.pid = pid; p.arg = arg; p.arg2 = arg2;
     for (int64_t i = 0; i < n; ++i) {
         Env s;
         uint16_t sb[kSlots] = {0};
         load_env<1>(s, sb, st, n, i);
-        int res = 0;
-        switch (phase) {
-        case INV_PHASE_TRY_MOVE: res = pid ? try_move(s, 1, arg) : try_move(s, 0, arg); break;
-        case INV_PHASE_SPAWN_BULLET: res = pid ? spawn_bullet<1>(s, sb, 1, arg, status) : spawn_bullet<1>(s, sb, 0, arg, status); break;
-        case INV_PHASE_WIDE_SHOT: res = pid ? spawn_wide_shot<1>(s, sb, 1, arg, status) : spawn_wide_shot<1>(s, sb, 0, arg, status); break;
-        case INV_PHASE_RELOAD: reload_ammo(s); break;
-        case INV_PHASE_UPDATE_BULLETS: update_bullets<1>(s, sb); break;
-        case INV_PHASE_STEP_PLAYERS: step_players<1>(s, sb, arg, arg2, status); break;
-        case INV_PHASE_ENGINE_RESET: {
-            s.episode += 1u;
-            Draws dr;
-            dr.init(p, env_id_base + (uint32_t)i, s.episode, INV_STREAM_RESET, nullptr);
-            engine_reset(s, dr);
-            break;
-        }
-        case INV_PHASE_DUMMY_POLICY: {
-            Draws dr;
-            dr.init(p, env_id_base + (uint32_t)i, s.episode, s.step, nullptr);
-            res = dummy_policy(s, dr, difficulty);
-            break;
-        }
-        default: return -1;
-        }
-        result[i] = (uint8_t)res;
+        result[i] = debug_phase<1>(s, sb, p, env_id_base + (uint32_t)i, nullptr);
         store_env<1>(s, sb, st, n, i);
+    }
+    return 0;
+}
+
+// Canonical state of envs [first, first+count) out of / into the planes, like inv_export_state /
+// inv_import_state (same conversions). The import writes nothing unless every env is in range.
+int hk_export_state(const uint32_t *planes, int64_t n, int64_t first, int64_t count, inv_env_state *out)
+{
+    for (int64_t k = 0; k < count; ++k) {
+        Env s;
+        uint16_t sb[kSlots];
+        load_env<1>(s, sb, reinterpret_cast<const uint4 *>(planes), n, first + k);
+        env_to_canonical(s, sb, out[k]);
+    }
+    return 0;
+}
+
+int hk_import_state(uint32_t *planes, int64_t n, int64_t first, int64_t count, const inv_env_state *in)
+{
+    Env s;
+    uint16_t sb[kSlots];
+    for (int64_t k = 0; k < count; ++k)
+        if (!env_from_canonical(in[k], s, sb)) return -1;
+    for (int64_t k = 0; k < count; ++k) {
+        env_from_canonical(in[k], s, sb);
+        store_env<1>(s, sb, reinterpret_cast<uint4 *>(planes), n, first + k);
     }
     return 0;
 }
@@ -136,7 +142,8 @@ int hk_observation(const uint32_t *planes, int64_t n, int64_t i, int viewer, flo
 // Sanitizer target: a self-contained random rollout (no reference involved), built with
 // -fsanitize=address,undefined, exercising every branch family (both modes and difficulties,
 // charge-heavy actions, auto-reset, timeouts) so that out-of-bounds indexing or UB in the shared
-// game logic aborts the test.
+// game logic aborts the test. Every 20 steps all envs go through export and re-import, which must
+// leave the planes byte-identical.
 #include <cstdio>
 #include <vector>
 int main()
@@ -148,7 +155,9 @@ int main()
     for (int mode = 0; mode < 2; ++mode)
         for (int diff = 0; diff < 2; ++diff) {
             std::vector<uint32_t> planes((size_t)n * 20, 0u);
-            for (int64_t i = 0; i < n; ++i) planes[(size_t)(2 * n + i) * 4] = 0xFFFFFFFFu; // episode = none yet
+            std::vector<inv_env_state> states(n);
+            for (auto &e : states) e.episode = 0xFFFFFFFFu; // no episode yet
+            hk_import_state(planes.data(), n, 0, n, states.data());
             std::vector<float> obs1((size_t)n * INV_OBS_ELEMS), ex1((size_t)n * 4), obs2((size_t)n * INV_OBS_ELEMS), ex2((size_t)n * 4);
             std::vector<float> rew(n);
             std::vector<uint8_t> done(n), info(n);
@@ -169,6 +178,14 @@ int main()
                         (t / 50) % 2, 7, 1000, obs1.data(), ex1.data(), obs2.data(), ex2.data(), rew.data(),
                         done.data(), info.data(), steps.data(), ret.data(), &status);
                 for (int64_t i = 0; i < n; ++i) episodes += done[i];
+                if (t % 20 == 19) {
+                    const std::vector<uint32_t> before = planes;
+                    hk_export_state(planes.data(), n, 0, n, states.data());
+                    if (hk_import_state(planes.data(), n, 0, n, states.data()) != 0 || planes != before) {
+                        std::printf("export/import round trip changed the planes at step %d\n", t);
+                        return 1;
+                    }
+                }
                 if (t % 50 == 49) { // manual resets of a scattered index list
                     std::vector<int64_t> idx;
                     for (int64_t i = 0; i < n; i += 3) idx.push_back(i);

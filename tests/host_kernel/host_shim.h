@@ -28,14 +28,5 @@ static inline int __popc(uint32_t v) { return __builtin_popcount(v); }
 static inline double __dadd_rn(double a, double b) { return a + b; }
 static inline double __dmul_rn(double a, double b) { return a * b; }
 static inline float __double2float_rn(double a) { return (float)a; }
-static inline double __hiloint2double(int hi, int lo)
-{
-    const uint64_t bits = ((uint64_t)(uint32_t)hi << 32) | (uint32_t)lo;
-    double d;
-    memcpy(&d, &bits, 8);
-    return d;
-}
-static inline int __double2loint(double d) { uint64_t b; memcpy(&b, &d, 8); return (int)(uint32_t)b; }
-static inline int __double2hiint(double d) { uint64_t b; memcpy(&b, &d, 8); return (int)(uint32_t)(b >> 32); }
 static inline uint32_t atomicOr(uint32_t *p, uint32_t v) { const uint32_t o = *p; *p |= v; return o; }
 using std::abs;

@@ -343,31 +343,11 @@ def test_indexed_reset_for_every_observation_dtype(dtype):
 
 
 def test_state_import_export_roundtrip_and_validation():
+    from backends import check_state_import_export
     from inversus_b200 import BatchedInversus
     s = BatchedInversus(64, "dummy", "hard", 500, seed=1)
     s.reset()
-    st = s.export_state()
-    st["bullets"][3, :2] = [[4, 5, 1, 0], [9, 2, 3, 1]]
-    st["n_bullets"][3] = 2
-    st["episode_return"][3] = -1.2345678901234567
-    st["p1"][3] = (14, 9, 0, 29, 0)
-    s.import_state(st[3:4], first=10)
-    back = s.export_state(10, 1)
-    for f in st.dtype.names:
-        assert np.array_equal(back[f][0], st[f][3]), f
-    for field, bad in (("p1", (15, 0, 0, 0, 1)), ("p2", (0, 10, 0, 0, 1)), ("p1", (0, 0, 8, 0, 1)), ("p1", (0, 0, 0, 0, 2))):
-        x = st[:1].copy()
-        x[field][0] = bad
-        with pytest.raises(ValueError):
-            s.import_state(x)
-    x = st[:1].copy()
-    x["n_bullets"][0] = 17
-    with pytest.raises(ValueError):
-        s.import_state(x)
-    x = st[:1].copy()
-    x["tiles"][0][4] = 1 << 22  # bit beyond the 150 tiles
-    with pytest.raises(ValueError):
-        s.import_state(x)
+    check_state_import_export(s.export_state, s.import_state)
 
 
 def test_two_devices_in_one_process():

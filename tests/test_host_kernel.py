@@ -1,12 +1,15 @@
 """The product's OWN game logic on the CPU: the device functions of csrc/inversus_kernels.cuh
-(load_env / rl_step / rl_reset / build_row / store_env, everything except the kernel shell) are
-compiled for the host through tests/host_kernel/host_shim.h and
+(load_env / rl_step / rl_reset / debug_phase / build_row / store_env, everything except the kernel
+shell) and the canonical-state conversions of inv_export_state / inv_import_state are compiled for
+the host through tests/host_kernel/host_shim.h and
 
   * replayed against every committed golden fixture of the live Python reference -- the same
-    bit-exact bar as the GPU parity tests, but runnable without a GPU, and
-  * run under AddressSanitizer + UBSan on a random rollout (compute-sanitizer is closed on the
-    GPU pool, so this is the memory-safety check of the shared logic: bullet slots, tile words,
-    observation rows).
+    bit-exact bar as the GPU parity tests, but runnable without a GPU, with the state read back
+    through the product's own export,
+  * driven through the reference's own engine unit tests and the state import/export checks, and
+  * run under AddressSanitizer + UBSan on a random rollout that also round-trips every env through
+    export and import (compute-sanitizer is closed on the GPU pool, so this is the memory-safety
+    check of the shared logic: bullet slots, tile words, observation rows, state conversion).
 
 This is a test harness, not a fallback: nothing in the product can reach it (INV_HOST_BUILD is
 defined only by tests/host_kernel/harness.cpp)."""
@@ -16,7 +19,7 @@ import subprocess
 import numpy as np
 import pytest
 
-from backends import HostKernelBackend
+from backends import HostKernelBackend, check_state_import_export
 from golden.scenarios import SCENARIOS, compare, run_scenario
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -46,6 +49,12 @@ def test_kernel_logic_under_address_and_ub_sanitizers(tmp_path):
                        env=dict(os.environ, ASAN_OPTIONS="detect_leaks=0"))
     assert r.returncode == 0, r.stdout[-1000:] + r.stderr[-3000:]
     assert "sanitizer run ok" in r.stdout
+
+
+def test_state_import_export_roundtrip_and_validation_on_host():
+    b = HostKernelBackend(dict(n=64, mode="dummy", difficulty="hard", max_steps=500, seed=1))
+    b.reset(None)
+    check_state_import_export(b.export_state, b.import_state)
 
 
 import reference_kat as K  # noqa: E402
