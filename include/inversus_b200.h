@@ -308,6 +308,32 @@ int inv_conv3x3_wgrad(const void *dy, const void *x, int64_t B, int32_t cin, int
 int inv_transpose_cast(const void *src, int32_t src_is_f32, int64_t ld_src, void *dst, int32_t dst_is_f32,
                        int64_t ld_dst, int64_t rows, int32_t A, int32_t B, void *stream);
 
+/* The evaluator's two device steps (csrc/eval_kernels.cu; DESIGN.md "evaluator"). Handle-free like
+ * inv_encode_fwd: one launch on `stream` on the current device, capturable in a CUDA graph.
+ * packed_dev / stride: [5, stride] uint4 planes (a view of INV_BUF_PACKED_STATE), entries [0, count).
+ *
+ * inv_select_actions: logits [count, 13] fp32 (contiguous rows) -> actions_out [count] int8.
+ *   greedy != 0: the first index of the maximum (torch.argmax). greedy == 0: one Philox4x32-10 draw r,
+ *   key = seed, counter = (gid_base + i, episode, step_count, 0x80000000 | seat), the env's pre-step
+ *   counter words; inverse CDF in fp32: m = max, e_j = expf(l_j - m), S = e_0 + ... + e_12 in order,
+ *   the smallest j with (r * 2^-32) * S < e_0 + ... + e_j, else the last j with e_j > 0. seat: 0 or 1.
+ *   packed_dev may be NULL when greedy. A row holding NaN or +inf, or only -inf, gets id -1, which
+ *   the next inv_step reports as INV_STATUS_INVALID_ACTION.
+ *
+ * inv_episode_tally: call after each inv_step of an auto-reset handle with its done / info /
+ *   episode_steps / episode_return buffers and its post-step packed state. An env whose episode with
+ *   index (episode - 1) ended in the step and whose index is < quota adds into its column of
+ *   counts_dev int32 [4][count] (wins, losses, draws = done with neither INV_INFO_WIN nor
+ *   INV_INFO_LOSE, sum of episode lengths) and return_sum_dev f64 [count] (summed in step order).
+ *   remaining_dev (one int32) is zeroed and then receives the number of envs whose post-step
+ *   episode is < quota. quota * max_episode_steps must be below 2^31. */
+int inv_select_actions(const float *logits, int64_t count, const void *packed_dev, int64_t stride, int64_t gid_base,
+                       uint64_t seed, int seat, int greedy, int8_t *actions_out, void *stream);
+int inv_episode_tally(const uint8_t *done, const uint8_t *info, const int32_t *episode_steps,
+                      const double *episode_return, const void *packed_dev, int64_t stride, int64_t count, int64_t quota,
+                      int32_t max_episode_steps, int32_t *counts_dev, double *return_sum_dev, int32_t *remaining_dev,
+                      void *stream);
+
 /* kernel launches issued through this handle so far (bench.py's gpu_launches) */
 int64_t inv_launch_count(const inv_sim *sim);
 

@@ -8,6 +8,7 @@ Public surface
     MultiEnvRunner, SingleInversusRLEnv, discrete_to_action   reference-shaped numpy API
     BatchedInversus                                           tensor-native API (device views)
     InversusCNNPolicy, PPOAgent, DeviceRollout, train_*       GPU-resident PPO around it (next rows)
+    evaluate                                                  K episodes per env vs the dummy or another policy
     shard_range, reduce_rollout_stats                         multi-GPU layout helpers
     build_library, library_path                               in-tree nvcc build of the C-ABI .so
 """
@@ -18,7 +19,7 @@ from ._capi import InversusError, library_path
 __all__ = ["constants", "build_library", "library_path", "InversusError", "BatchedInversus",
            "MultiEnvRunner", "SingleInversusRLEnv", "discrete_to_action", "build_observation", "PlayerId", "InfoList",
            "shard_range", "reduce_rollout_stats", "InversusCNNPolicy", "make_policy_from_env", "PPOAgent",
-           "DeviceRollout", "compute_gae", "train_vs_dummy", "train_selfplay"]
+           "DeviceRollout", "compute_gae", "train_vs_dummy", "train_selfplay", "evaluate"]
 
 _LAZY = {
     "BatchedInversus": ("simulator", "BatchedInversus"),
@@ -35,6 +36,7 @@ _LAZY = {
     "compute_gae": ("ppo_agent", "compute_gae"),
     "train_vs_dummy": ("training", "train_vs_dummy"),
     "train_selfplay": ("training", "train_selfplay"),
+    "evaluate": ("evaluate", "evaluate"),
     "shard_range": ("sharding", "shard_range"),
     "reduce_rollout_stats": ("sharding", "reduce_rollout_stats"),
 }
@@ -44,5 +46,8 @@ def __getattr__(name):  # lazy, like the reference's inversus_rl/__init__.py, so
     if name in _LAZY:
         import importlib
         mod, attr = _LAZY[name]
-        return getattr(importlib.import_module(f"{__name__}.{mod}"), attr)
+        value = getattr(importlib.import_module(f"{__name__}.{mod}"), attr)
+        if name == mod:  # importing the submodule bound its name here: keep the function instead
+            globals()[name] = value
+        return value
     raise AttributeError(f"module {__name__!r} has no attribute {name!r}")

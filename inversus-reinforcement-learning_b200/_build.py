@@ -9,7 +9,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_PATH = os.path.join(HERE, "libinversus_b200.so")
 SOURCES = [os.path.join(CSRC, "inversus_b200.cu"), os.path.join(CSRC, "policy_kernels.cu"),
-           os.path.join(CSRC, "encoder_kernels.cu"), os.path.join(CSRC, "wgrad_kernels.cu")]
+           os.path.join(CSRC, "encoder_kernels.cu"), os.path.join(CSRC, "wgrad_kernels.cu"),
+           os.path.join(CSRC, "eval_kernels.cu")]
 HOST_SOURCES = [os.path.join(CSRC, "host_expand.cpp")]  # plain C++ (AVX2 intrinsics), compiled by g++
 DEPS = SOURCES + HOST_SOURCES + [os.path.join(CSRC, "inversus_kernels.cuh"),
                   os.path.join(os.path.dirname(HERE), "include", "inversus_b200.h")]

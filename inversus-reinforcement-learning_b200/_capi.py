@@ -91,6 +91,9 @@ SYMBOLS = {
     "inv_conv3x3_wgrad": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "inv_gae": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_double, C.c_double, C.c_int32,
                           C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "inv_select_actions": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_uint64, C.c_int,
+                                     C.c_int, C.c_void_p, C.c_void_p]),
+    "inv_episode_tally": (C.c_int, [C.c_void_p] * 5 + [C.c_int64, C.c_int64, C.c_int64, C.c_int32] + [C.c_void_p] * 4),
 }
 
 _lib = None

@@ -72,6 +72,10 @@ static int fail(int code, const char *fmt, const char *a = "", const char *b = "
     return code;
 }
 
+namespace inv_host { // the handle-free entry points of eval_kernels.cu report through the same text
+int set_error(int code, const char *who, const char *msg) { return fail(code, "%s: %s", who, msg); }
+} // namespace inv_host
+
 #define CUDA_TRY(expr)                                                                      \
     do {                                                                                    \
         cudaError_t e_ = (expr);                                                            \

@@ -202,6 +202,17 @@ INV_HD uint32_t double_hi_word(double d)
 #endif
 }
 
+// The two RNG counter words of an env, (step_count, episode), from its planes 1 and 2. Consumers
+// that need only the counters (the evaluator's action selector and episode tally) read them here.
+struct Counters {
+    uint32_t step, episode;
+};
+INV_HD Counters counters_from_planes(const uint4 &b, const uint4 &c) { return Counters{b.w, c.x}; }
+INV_HD Counters load_counters(const uint4 *st, int64_t stride, int64_t i)
+{
+    return counters_from_planes(st[stride + i], st[2 * stride + i]);
+}
+
 template <int E>
 INV_HD void load_env(Env &s, uint16_t *sb, const uint4 *st, int64_t stride, int64_t i)
 {
@@ -211,8 +222,9 @@ INV_HD void load_env(Env &s, uint16_t *sb, const uint4 *st, int64_t stride, int6
     unpack_player(s, 0, b.y);
     s.nb = (int)(b.y >> 20) & 31;
     unpack_player(s, 1, b.z);
-    s.step = b.w;
-    s.episode = c.x;
+    const Counters k = counters_from_planes(b, c);
+    s.step = k.step;
+    s.episode = k.episode;
     s.ret = double_from_words(c.y, c.z);
     const uint32_t w[8] = {d.x, d.y, d.z, d.w, e.x, e.y, e.z, e.w};
 #pragma unroll

@@ -31,6 +31,36 @@ def dist_env() -> Tuple[int, int, int]:
             int(os.environ.get("WORLD_SIZE", 1)))
 
 
+def init_distributed() -> Tuple[int, int, int]:
+    """Join the NCCL process group when started by torchrun with more than one process (one GPU each)."""
+    rank, local_rank, world = dist_env()
+    if world > 1 and not torch.distributed.is_initialized():
+        os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
+        torch.cuda.set_device(local_rank)
+        torch.distributed.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
+    return rank, local_rank, world
+
+
+def finish_distributed() -> None:
+    """End a torchrun command-line run (no-op without a process group). CUDA graphs may hold NCCL
+    kernels: drop them, then give the communicator teardown a bounded time on a side thread (it has
+    been seen to block with captured collectives) and leave."""
+    if not torch.distributed.is_initialized():
+        return
+    import gc
+    import sys
+    import threading
+    gc.collect()
+    torch.cuda.synchronize()
+    torch.distributed.barrier()
+    t = threading.Thread(target=torch.distributed.destroy_process_group, daemon=True)
+    t.start()
+    t.join(20.0)
+    sys.stdout.flush()
+    sys.stderr.flush()
+    os._exit(0)
+
+
 def reduce_rollout_stats(episodes, wins, return_sum, length_sum, device=None) -> Tuple[float, float, float, float]:
     """Sum the four rollout statistics over ranks (no-op without an initialised process group)."""
     t = torch.tensor([float(episodes), float(wins), float(return_sum), float(length_sum)],

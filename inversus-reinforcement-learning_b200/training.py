@@ -26,7 +26,7 @@ import torch
 from .constants import INFO_WIN
 from .policies import InversusCNNPolicy
 from .ppo_agent import DeviceRollout, PPOAgent
-from .sharding import dist_env, reduce_rollout_stats, shard_range
+from .sharding import dist_env, finish_distributed, init_distributed, reduce_rollout_stats, shard_range
 from .simulator import BatchedInversus
 
 OPPONENT_UPDATE_FREQ = 20000  # training.py:265
@@ -57,15 +57,6 @@ class TrainingLogger:
             csv.writer(f).writerow([step, elapsed, samples_per_s, rollout_rate, update_s])
 
 
-def _init_distributed():
-    rank, local_rank, world = dist_env()
-    if world > 1 and not torch.distributed.is_initialized():
-        os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
-        torch.cuda.set_device(local_rank)
-        torch.distributed.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
-    return rank, local_rank, world
-
-
 def train(mode: str = "vs_dummy", num_envs: int = 1, total_steps: int = 500_000, log_dir: Optional[str] = None,
           opponent_difficulty: str = "easy", load_model: Optional[str] = None, *, precision: str = "bf16",
           rollout_steps: Optional[int] = None, batch_size: Optional[int] = None, epochs: int = 4, lr: float = 1e-4,
@@ -76,7 +67,7 @@ def train(mode: str = "vs_dummy", num_envs: int = 1, total_steps: int = 500_000,
     torchrun each rank simulates its shard. Returns a summary dict (steps, episodes, win_rate,
     samples_per_s, ...)."""
     assert mode in ("vs_dummy", "selfplay")
-    rank, local_rank, world = _init_distributed()
+    rank, local_rank, world = init_distributed()
     dev = torch.device("cuda", local_rank if world > 1 else torch.cuda.current_device())
     first, n_local = shard_range(num_envs, rank, world)
     log_dir = log_dir or f"runs/inversus_{mode}_envs{num_envs}"
@@ -340,21 +331,7 @@ def main(argv=None):
                 cuda_graph={"auto": None, "on": True, "off": False}[a.cuda_graph])
     if dist_env()[0] == 0:
         print({k: (round(v, 4) if isinstance(v, float) else v) for k, v in out.items()}, flush=True)
-    if torch.distributed.is_initialized():
-        # the update graph holds NCCL kernels: drop it, then give the communicator teardown a bounded
-        # time on a side thread (it has been seen to block with captured collectives) and leave
-        import gc
-        import sys
-        import threading
-        gc.collect()
-        torch.cuda.synchronize()
-        torch.distributed.barrier()
-        t = threading.Thread(target=torch.distributed.destroy_process_group, daemon=True)
-        t.start()
-        t.join(20.0)
-        sys.stdout.flush()
-        sys.stderr.flush()
-        os._exit(0)
+    finish_distributed()  # the update graph holds NCCL kernels
 
 
 if __name__ == "__main__":
