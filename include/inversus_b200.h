@@ -12,6 +12,10 @@
  * Conventions
  *   - Every function returns an inv_status code (0 = INV_OK); inv_last_error() gives the text of
  *     the calling thread's last failure.
+ *   - There is no CPU fallback: every compute entry point fails with INV_ERR_NO_DEVICE unless its
+ *     device (the handle's; the current one for handle-free calls) is an sm_100 part. The scratch-size
+ *     queries (inv_ln_relu_partials, inv_encode_partials_floats, inv_conv3x3_wgrad_scratch_floats) and
+ *     the inv_host_* calls run anywhere.
  *   - `stream` is a cudaStream_t passed as void* (NULL = legacy default stream). Calls enqueue
  *     work and return; nothing synchronises unless stated. One handle per GPU; a handle is not
  *     thread-safe.
@@ -308,8 +312,8 @@ int inv_conv3x3_wgrad(const void *dy, const void *x, int64_t B, int32_t cin, int
 int inv_transpose_cast(const void *src, int32_t src_is_f32, int64_t ld_src, void *dst, int32_t dst_is_f32,
                        int64_t ld_dst, int64_t rows, int32_t A, int32_t B, void *stream);
 
-/* The evaluator's two device steps (csrc/eval_kernels.cu; DESIGN.md "evaluator"). Handle-free like
- * inv_encode_fwd: one launch on `stream` on the current device, capturable in a CUDA graph.
+/* The evaluator's two device steps (csrc/eval_kernels.cu; DESIGN.md "evaluator"). Handle-free: one
+ * launch on `stream` on the current device, capturable in a CUDA graph.
  * packed_dev / stride: [5, stride] uint4 planes (a view of INV_BUF_PACKED_STATE), entries [0, count).
  *
  * inv_select_actions: logits [count, 13] fp32 (contiguous rows) -> actions_out [count] int8.

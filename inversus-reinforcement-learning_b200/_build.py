@@ -12,7 +12,7 @@ SOURCES = [os.path.join(CSRC, "inversus_b200.cu"), os.path.join(CSRC, "policy_ke
            os.path.join(CSRC, "encoder_kernels.cu"), os.path.join(CSRC, "wgrad_kernels.cu"),
            os.path.join(CSRC, "eval_kernels.cu")]
 HOST_SOURCES = [os.path.join(CSRC, "host_expand.cpp")]  # plain C++ (AVX2 intrinsics), compiled by g++
-DEPS = SOURCES + HOST_SOURCES + [os.path.join(CSRC, "inversus_kernels.cuh"),
+DEPS = SOURCES + HOST_SOURCES + [os.path.join(CSRC, "inversus_kernels.cuh"), os.path.join(CSRC, "launch_common.h"),
                   os.path.join(os.path.dirname(HERE), "include", "inversus_b200.h")]
 
 # --cudart=shared: the artefact links libcudart dynamically instead of embedding the whole runtime

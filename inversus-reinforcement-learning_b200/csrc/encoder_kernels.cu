@@ -25,6 +25,7 @@
 #include <stdint.h>
 
 #include "../../include/inversus_b200.h"
+#include "launch_common.h"
 
 namespace {
 
@@ -472,80 +473,58 @@ __global__ void encode_reduce_kernel(const float *__restrict__ red, float *__res
     if (k < kCo) db1[k] = total(dense0 + 9 * kCo + k);
 }
 
-int sm_count_enc()
-{
-    static int n[64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64) return 148;
-    if (n[dev] == 0) {
-        cudaDeviceGetAttribute(&n[dev], cudaDevAttrMultiProcessorCount, dev);
-        if (n[dev] <= 0) n[dev] = 148;
-    }
-    return n[dev];
-}
-
 constexpr size_t kFwdSmem = sizeof(Tables) + (size_t)kFwdWarps * kD * 2;
 constexpr size_t kBwdSmem = sizeof(Tables) + (size_t)kBwdWarps * kD * 2 + (size_t)kBwdWarps * kSparse * 9 * kCo * 4;
+constexpr const char *kBadArg = "null pointer, count or stride out of range, or view not 0 or 1";
 
 } // namespace
 
 extern "C" {
 
-int inv_encode_partials_floats(void) { return (sm_count_enc() + 1) * kPartial; } // per-CTA partials + their sum
+int inv_encode_partials_floats(void) { return (inv_host::sm_count() + 1) * kPartial; } // per-CTA partials + their sum
 
 int inv_encode_fwd(const void *packed_dev, int64_t stride, int64_t count, int view, const float *w1, const float *b1,
                    const float *gamma_hwc, const float *beta_hwc, float eps, void *y_out, float *extra_out,
                    float *mean_out, float *rstd_out, void *stream)
 {
+    const char *who = "inv_encode_fwd";
+    if (int rc = inv_host::require_sm100(who)) return rc;
     if (!packed_dev || !w1 || !b1 || !gamma_hwc || !beta_hwc || !y_out || !mean_out || !rstd_out || count < 0 ||
         stride < count || (view != 0 && view != 1))
-        return INV_ERR_INVALID_ARG;
+        return inv_host::set_error(INV_ERR_INVALID_ARG, who, kBadArg);
     if (count == 0) return INV_OK;
-    static bool configured[64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !configured[dev]) {
-        if (cudaFuncSetAttribute(encode_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmem) != cudaSuccess)
-            return INV_ERR_CUDA;
-        if (dev >= 0 && dev < 64) configured[dev] = true;
-    }
-    const int64_t want = (count + kFwdWarps - 1) / kFwdWarps;
-    const unsigned grid = (unsigned)(want < sm_count_enc() ? want : sm_count_enc());
+    if (inv_host::allow_dynamic_smem((const void *)encode_fwd_kernel, kFwdSmem) != cudaSuccess) return inv_host::launch_status(who);
+    const int64_t want = (count + kFwdWarps - 1) / kFwdWarps, nsm = inv_host::sm_count();
+    const unsigned grid = (unsigned)(want < nsm ? want : nsm);
     encode_fwd_kernel<<<grid, kFwdWarps * 32, kFwdSmem, (cudaStream_t)stream>>>(
         static_cast<const uint32_t *>(packed_dev), stride, count, view, w1, b1, reinterpret_cast<const float2 *>(gamma_hwc),
         reinterpret_cast<const float2 *>(beta_hwc), eps, static_cast<uint32_t *>(y_out),
         reinterpret_cast<float4 *>(extra_out), mean_out, rstd_out);
-    return cudaGetLastError() == cudaSuccess ? INV_OK : INV_ERR_CUDA;
+    return inv_host::launch_status(who);
 }
 
 int inv_encode_bwd(const void *packed_dev, int64_t stride, int64_t count, int view, const float *w1, const float *b1,
                    const float *gamma_hwc, const float *beta_hwc, const float *mean, const float *rstd, const void *dy,
                    float *dw1, float *db1, float *dgamma_hwc, float *dbeta_hwc, float *partials, void *stream)
 {
+    const char *who = "inv_encode_bwd";
+    if (int rc = inv_host::require_sm100(who)) return rc;
     if (!packed_dev || !w1 || !b1 || !gamma_hwc || !beta_hwc || !mean || !rstd || !dy || !dw1 || !db1 || !dgamma_hwc ||
         !dbeta_hwc || !partials || count <= 0 || stride < count || (view != 0 && view != 1))
-        return INV_ERR_INVALID_ARG;
-    static bool configured[64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !configured[dev]) {
-        if (cudaFuncSetAttribute(encode_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBwdSmem) != cudaSuccess)
-            return INV_ERR_CUDA;
-        if (dev >= 0 && dev < 64) configured[dev] = true;
-    }
-    const int64_t want = (count + kBwdWarps - 1) / kBwdWarps;
-    const int grid = (int)(want < sm_count_enc() ? want : sm_count_enc());
+        return inv_host::set_error(INV_ERR_INVALID_ARG, who, kBadArg);
+    if (inv_host::allow_dynamic_smem((const void *)encode_bwd_kernel, kBwdSmem) != cudaSuccess) return inv_host::launch_status(who);
+    const int64_t want = (count + kBwdWarps - 1) / kBwdWarps, nsm = inv_host::sm_count();
+    const int grid = (int)(want < nsm ? want : nsm);
     cudaStream_t st = (cudaStream_t)stream;
     encode_bwd_kernel<<<grid, kBwdWarps * 32, kBwdSmem, st>>>(
         static_cast<const uint32_t *>(packed_dev), stride, count, view, w1, b1, reinterpret_cast<const float2 *>(gamma_hwc),
         reinterpret_cast<const float2 *>(beta_hwc), mean, rstd, static_cast<const uint32_t *>(dy), partials);
-    if (cudaGetLastError() != cudaSuccess) return INV_ERR_CUDA;
-    float *red = partials + (size_t)sm_count_enc() * kPartial;
+    if (int rc = inv_host::launch_status(who)) return rc;
+    float *red = partials + (size_t)nsm * kPartial;
     encode_sum_partials_kernel<<<(kPartial + 31) / 32, dim3(32, 8), 0, st>>>(partials, grid, red);
     const int outputs = 2 * kD + kCo * kCi * 9 + kCo;
     encode_reduce_kernel<<<(outputs + 127) / 128, 128, 0, st>>>(red, dw1, db1, dgamma_hwc, dbeta_hwc);
-    return cudaGetLastError() == cudaSuccess ? INV_OK : INV_ERR_CUDA;
+    return inv_host::launch_status(who);
 }
 
 } // extern "C"

@@ -13,40 +13,15 @@
 // owner thread; the only atomic adds an integer count into `remaining`, whose sum does not depend
 // on the order of the additions.
 #include "inversus_kernels.cuh"
+#include "launch_common.h"
 
 using namespace inv;
-
-namespace inv_host { // inversus_b200.cu: the thread-local text behind inv_last_error()
-int set_error(int code, const char *who, const char *msg);
-} // namespace inv_host
 
 namespace {
 
 constexpr int kA = INV_NUM_ACTIONS;
 constexpr int kSelThreads = 256;
 constexpr int kTallyThreads = 256;
-
-// INV_OK when the current device is an sm_100 part; otherwise the same error as inv_create
-int require_sm100(const char *who)
-{
-    static int major[64] = {};
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        return inv_host::set_error(INV_ERR_NO_DEVICE, who, "no CUDA device: this simulator has no CPU fallback");
-    }
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) return inv_host::set_error(INV_ERR_CUDA, who, "cudaGetDevice failed");
-    int m = (dev >= 0 && dev < 64) ? major[dev] : 0;
-    if (m == 0) {
-        if (cudaDeviceGetAttribute(&m, cudaDevAttrComputeCapabilityMajor, dev) != cudaSuccess)
-            return inv_host::set_error(INV_ERR_CUDA, who, "cudaDeviceGetAttribute failed");
-        if (dev >= 0 && dev < 64) major[dev] = m;
-    }
-    if (m != 10)
-        return inv_host::set_error(INV_ERR_NO_DEVICE, who, "device is not sm_100 (B200): kernels are built for sm_100a only");
-    return INV_OK;
-}
 
 // One thread per row. The block's rows are staged through shared memory so that the global reads
 // are coalesced; a row's 13 floats then sit at an odd word stride, which is bank-conflict free.
@@ -138,7 +113,7 @@ int inv_select_actions(const float *logits, int64_t count, const void *packed_de
                        uint64_t seed, int seat, int greedy, int8_t *actions_out, void *stream)
 {
     const char *who = "inv_select_actions";
-    if (int rc = require_sm100(who)) return rc;
+    if (int rc = inv_host::require_sm100(who)) return rc;
     if (count < 0 || !logits || !actions_out || (!greedy && (!packed_dev || stride < count)) || (seat != 0 && seat != 1) ||
         gid_base < 0 || gid_base > 0x100000000ll - count)
         return inv_host::set_error(INV_ERR_INVALID_ARG, who, "bad argument");
@@ -147,8 +122,7 @@ int inv_select_actions(const float *logits, int64_t count, const void *packed_de
     select_actions_kernel<<<(unsigned)blocks, kSelThreads, 0, (cudaStream_t)stream>>>(
         logits, count, static_cast<const uint4 *>(packed_dev), stride, (uint32_t)gid_base, (uint32_t)seed,
         (uint32_t)(seed >> 32), (uint32_t)seat, greedy, actions_out);
-    const cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? INV_OK : inv_host::set_error(INV_ERR_CUDA, who, cudaGetErrorString(e));
+    return inv_host::launch_status(who);
 }
 
 int inv_episode_tally(const uint8_t *done, const uint8_t *info, const int32_t *episode_steps,
@@ -157,7 +131,7 @@ int inv_episode_tally(const uint8_t *done, const uint8_t *info, const int32_t *e
                       void *stream)
 {
     const char *who = "inv_episode_tally";
-    if (int rc = require_sm100(who)) return rc;
+    if (int rc = inv_host::require_sm100(who)) return rc;
     if (count < 0 || !done || !info || !episode_steps || !episode_return || !packed_dev || stride < count || !counts_dev ||
         !return_sum_dev || !remaining_dev || max_episode_steps <= 0)
         return inv_host::set_error(INV_ERR_INVALID_ARG, who, "bad argument");
@@ -165,15 +139,13 @@ int inv_episode_tally(const uint8_t *done, const uint8_t *info, const int32_t *e
         return inv_host::set_error(INV_ERR_INVALID_ARG, who,
                                    "quota * max_episode_steps must be below 2^31 (the per-env length sum is int32)");
     cudaStream_t st = (cudaStream_t)stream;
-    cudaError_t e = cudaMemsetAsync(remaining_dev, 0, sizeof(int32_t), st);
-    if (e == cudaSuccess && count > 0) {
-        const int64_t blocks = (count + kTallyThreads - 1) / kTallyThreads;
-        episode_tally_kernel<<<(unsigned)blocks, kTallyThreads, 0, st>>>(
-            done, info, episode_steps, episode_return, static_cast<const uint4 *>(packed_dev), stride, count,
-            (uint32_t)quota, counts_dev, return_sum_dev, remaining_dev);
-        e = cudaGetLastError();
-    }
-    return e == cudaSuccess ? INV_OK : inv_host::set_error(INV_ERR_CUDA, who, cudaGetErrorString(e));
+    if (cudaMemsetAsync(remaining_dev, 0, sizeof(int32_t), st) != cudaSuccess) return inv_host::launch_status(who);
+    if (count == 0) return INV_OK;
+    const int64_t blocks = (count + kTallyThreads - 1) / kTallyThreads;
+    episode_tally_kernel<<<(unsigned)blocks, kTallyThreads, 0, st>>>(
+        done, info, episode_steps, episode_return, static_cast<const uint4 *>(packed_dev), stride, count,
+        (uint32_t)quota, counts_dev, return_sum_dev, remaining_dev);
+    return inv_host::launch_status(who);
 }
 
 } // extern "C"

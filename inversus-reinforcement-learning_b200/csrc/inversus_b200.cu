@@ -5,23 +5,18 @@
 // third-party code: CUDA runtime only. There is deliberately no CPU fallback -- every entry point
 // fails with INV_ERR_NO_DEVICE / INV_ERR_CUDA when no sm_100 device is usable.
 #include "inversus_kernels.cuh"
+#include "launch_common.h"
 
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <mutex>
 #include <new>
 #include <thread>
 #include <vector>
 
 using namespace inv;
-
-namespace inv_host { // host_expand.cpp
-void expand_f32(const uint32_t *bits, float *dst, int64_t lo, int64_t hi, int nthreads);
-int hardware_threads();
-bool stage_action_ids(int8_t *dst, const int8_t *src, int64_t n);
-bool check_action_ids(const int8_t *src, int64_t n);
-} // namespace inv_host
 
 struct inv_sim {
     inv_config cfg;
@@ -34,7 +29,6 @@ struct inv_sim {
     double *ep_return, *reward64;
     uint32_t *status;
     const uint32_t *table;
-    int sm_count;
     int64_t launches;
     bool was_reset;
     // staging for the *_host calls: pinned host + device copies of the action ids
@@ -72,8 +66,69 @@ static int fail(int code, const char *fmt, const char *a = "", const char *b = "
     return code;
 }
 
-namespace inv_host { // the handle-free entry points of eval_kernels.cu report through the same text
+namespace inv_host { // launch_common.h
 int set_error(int code, const char *who, const char *msg) { return fail(code, "%s: %s", who, msg); }
+
+int require_sm100(const char *who)
+{
+    static int major[64] = {};
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
+        cudaGetLastError();
+        return set_error(INV_ERR_NO_DEVICE, who, "no CUDA device: this simulator has no CPU fallback");
+    }
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess) return set_error(INV_ERR_CUDA, who, "cudaGetDevice failed");
+    int m = (dev >= 0 && dev < 64) ? major[dev] : 0;
+    if (m == 0) {
+        if (cudaDeviceGetAttribute(&m, cudaDevAttrComputeCapabilityMajor, dev) != cudaSuccess)
+            return set_error(INV_ERR_CUDA, who, "cudaDeviceGetAttribute failed");
+        if (dev >= 0 && dev < 64) major[dev] = m;
+    }
+    return m == 10 ? INV_OK
+                   : set_error(INV_ERR_NO_DEVICE, who, "device is not sm_100 (B200): kernels are built for sm_100a only");
+}
+
+int sm_count()
+{
+    static int n[64] = {};
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (dev < 0 || dev >= 64) return 148;
+    if (n[dev] == 0) {
+        cudaDeviceGetAttribute(&n[dev], cudaDevAttrMultiProcessorCount, dev);
+        if (n[dev] <= 0) n[dev] = 148;
+    }
+    return n[dev];
+}
+
+cudaError_t allow_dynamic_smem(const void *kernel, size_t bytes)
+{
+    // the largest limit set so far per (kernel, device). The library has fewer than 100 kernels; any
+    // left out of a full table set the attribute on every call.
+    struct Limit { const void *kernel; int dev; size_t bytes; };
+    static Limit limits[256];
+    static int used = 0;
+    static std::mutex mu;
+    int dev = 0;
+    if (cudaError_t e = cudaGetDevice(&dev)) return e;
+    std::lock_guard<std::mutex> lock(mu);
+    int i = 0;
+    while (i < used && (limits[i].kernel != kernel || limits[i].dev != dev)) ++i;
+    if (i < used && limits[i].bytes >= bytes) return cudaSuccess;
+    const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    if (e == cudaSuccess && i < 256) {
+        limits[i] = Limit{kernel, dev, bytes};
+        if (i == used) ++used;
+    }
+    return e;
+}
+
+int launch_status(const char *who)
+{
+    const cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? INV_OK : set_error(INV_ERR_CUDA, who, cudaGetErrorString(e));
+}
 } // namespace inv_host
 
 #define CUDA_TRY(expr)                                                                      \
@@ -292,19 +347,11 @@ constexpr int kTileEnvs = 32;
 #endif
 
 template <int OP, int DT, bool P2V, bool INDEXED, int E, int T = kThreads>
-cudaError_t launch_one(const Params &p, int sm_count, cudaStream_t st)
+cudaError_t launch_one(const Params &p, cudaStream_t st)
 {
-    (void)sm_count;
     auto kern = inv_kernel<OP, DT, P2V, INDEXED, E, T>;
     constexpr size_t smem = smem_bytes<E, P2V, INDEXED, DT>();
-    static bool configured[64] = {}; // per instantiation and per device (function attributes are per device)
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !configured[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        if (dev >= 0 && dev < 64) configured[dev] = true;
-    }
+    if (cudaError_t e = inv_host::allow_dynamic_smem((const void *)kern, smem)) return e;
     const int64_t ntiles = (p.count + E - 1) / E;
     if (ntiles <= 0) return cudaSuccess;
     const unsigned grid = (unsigned)(ntiles < (int64_t)0x7FFFFFFF ? ntiles : (int64_t)0x7FFFFFFF);
@@ -313,33 +360,32 @@ cudaError_t launch_one(const Params &p, int sm_count, cudaStream_t st)
 }
 
 template <int OP, int DT, bool P2V, bool INDEXED>
-cudaError_t launch_e(const Params &p, int sm_count, cudaStream_t st)
+cudaError_t launch_e(const Params &p, cudaStream_t st)
 {
     if constexpr (DT == INV_OBS_NONE && !INDEXED && OP != OP_DEBUG) {
-        return launch_one<OP, DT, P2V, false, 128, 128>(p, sm_count, st); // pure thread-per-env, no store phase
+        return launch_one<OP, DT, P2V, false, 128, 128>(p, st); // pure thread-per-env, no store phase
     } else if constexpr (OP == OP_STEP && !INDEXED && DT != INV_OBS_F32) {
         constexpr int E = (DT == INV_OBS_BF16 && !P2V) ? INV_BF16_E : INV_NARROW_E;
         constexpr int T = (DT == INV_OBS_BF16 && !P2V) ? INV_BF16_T : INV_NARROW_T;
-        return launch_one<OP_STEP, DT, P2V, false, E, T>(p, sm_count, st);
+        return launch_one<OP_STEP, DT, P2V, false, E, T>(p, st);
     } else if constexpr (DT == INV_OBS_F32 && !INDEXED && OP != OP_DEBUG) {
         if (p.count >= INV_WIDE_MIN_ENVS) {
-            if constexpr (OP == OP_STEP && !P2V) return launch_one<OP, DT, P2V, false, 64, 256>(p, sm_count, st);
-            else if constexpr (OP == OP_STEP) return launch_one<OP, DT, P2V, false, 64, 384>(p, sm_count, st);
-            else return launch_one<OP, DT, P2V, false, 128, 512>(p, sm_count, st);
+            if constexpr (OP == OP_STEP && !P2V) return launch_one<OP, DT, P2V, false, 64, 256>(p, st);
+            else if constexpr (OP == OP_STEP) return launch_one<OP, DT, P2V, false, 64, 384>(p, st);
+            else return launch_one<OP, DT, P2V, false, 128, 512>(p, st);
         }
-        return launch_one<OP, DT, P2V, INDEXED, kTileEnvs>(p, sm_count, st);
+        return launch_one<OP, DT, P2V, INDEXED, kTileEnvs>(p, st);
     } else {
-        return launch_one<OP, DT, P2V, INDEXED, kTileEnvs>(p, sm_count, st);
+        return launch_one<OP, DT, P2V, INDEXED, kTileEnvs>(p, st);
     }
 }
 
 template <int OP, bool INDEXED>
-cudaError_t launch(const Params &p, int dt, bool p2v, int sm_count, cudaStream_t st)
+cudaError_t launch(const Params &p, int dt, bool p2v, cudaStream_t st)
 {
 #define INV_CASE(DTV)                                                                   \
     case DTV:                                                                           \
-        return p2v ? launch_e<OP, DTV, true, INDEXED>(p, sm_count, st)                  \
-                   : launch_e<OP, DTV, false, INDEXED>(p, sm_count, st);
+        return p2v ? launch_e<OP, DTV, true, INDEXED>(p, st) : launch_e<OP, DTV, false, INDEXED>(p, st);
     switch (dt) {
         INV_CASE(INV_OBS_F32)
         INV_CASE(INV_OBS_BF16)
@@ -394,7 +440,6 @@ int inv_create(const inv_config *cfg, inv_sim **out)
     s->cfg = *cfg;
     if (cfg->mode == INV_MODE_SELFPLAY) s->cfg.flags |= INV_FLAG_P2_VIEW; // env_wrappers.py:311
     s->n = cfg->n_envs;
-    s->sm_count = prop.multiProcessorCount;
     s->host_threads = inv_host::hardware_threads() > 32 ? 32 : inv_host::hardware_threads();
     s->dma_frac = 0.35;
     s->dma_frac_auto = true;
@@ -567,8 +612,7 @@ int inv_reset(inv_sim *s, void *stream)
     if (!s) return fail(INV_ERR_INVALID_ARG, "inv_reset: null handle");
     DeviceGuard g(s->cfg.device);
     Params p = base_params(s);
-    CUDA_TRY((launch<OP_RESET, false>(p, s->cfg.obs_dtype, (s->cfg.flags & INV_FLAG_P2_VIEW) != 0, s->sm_count,
-                                      (cudaStream_t)stream)));
+    CUDA_TRY((launch<OP_RESET, false>(p, s->cfg.obs_dtype, (s->cfg.flags & INV_FLAG_P2_VIEW) != 0, (cudaStream_t)stream)));
     note_launch(s, (cudaStream_t)stream);
     s->was_reset = true;
     return INV_OK;
@@ -583,8 +627,7 @@ int inv_reset_envs(inv_sim *s, const int64_t *idx_dev, int64_t count, void *stre
     Params p = base_params(s);
     p.idx = idx_dev;
     p.count = count;
-    CUDA_TRY((launch<OP_RESET, true>(p, s->cfg.obs_dtype, (s->cfg.flags & INV_FLAG_P2_VIEW) != 0, s->sm_count,
-                                     (cudaStream_t)stream)));
+    CUDA_TRY((launch<OP_RESET, true>(p, s->cfg.obs_dtype, (s->cfg.flags & INV_FLAG_P2_VIEW) != 0, (cudaStream_t)stream)));
     note_launch(s, (cudaStream_t)stream);
     return INV_OK;
 }
@@ -604,8 +647,7 @@ static int step_impl(inv_sim *s, const int8_t *a1, const int8_t *a2, void *strea
     p.bits1 = bits1;
     p.bits2 = bits2;
     if (first != 0 || count != s->n) p = chunk_params(p, first, count, obs_env_bytes(s->cfg.obs_dtype));
-    CUDA_TRY((launch<OP_STEP, false>(p, s->cfg.obs_dtype, (s->cfg.flags & INV_FLAG_P2_VIEW) != 0, s->sm_count,
-                                     (cudaStream_t)stream)));
+    CUDA_TRY((launch<OP_STEP, false>(p, s->cfg.obs_dtype, (s->cfg.flags & INV_FLAG_P2_VIEW) != 0, (cudaStream_t)stream)));
     note_launch(s, (cudaStream_t)stream);
     return INV_OK;
 }
@@ -1097,9 +1139,9 @@ int inv_obs_from_packed(inv_sim *s, const void *packed_dev, int64_t stride, int6
     p.table = nullptr;
     cudaError_t ce;
     switch (obs_dtype) {
-    case INV_OBS_F32: ce = launch_e<OP_OBS, INV_OBS_F32, false, false>(p, s->sm_count, (cudaStream_t)stream); break;
-    case INV_OBS_BF16: ce = launch_e<OP_OBS, INV_OBS_BF16, false, false>(p, s->sm_count, (cudaStream_t)stream); break;
-    case INV_OBS_U8: ce = launch_e<OP_OBS, INV_OBS_U8, false, false>(p, s->sm_count, (cudaStream_t)stream); break;
+    case INV_OBS_F32: ce = launch_e<OP_OBS, INV_OBS_F32, false, false>(p, (cudaStream_t)stream); break;
+    case INV_OBS_BF16: ce = launch_e<OP_OBS, INV_OBS_BF16, false, false>(p, (cudaStream_t)stream); break;
+    case INV_OBS_U8: ce = launch_e<OP_OBS, INV_OBS_U8, false, false>(p, (cudaStream_t)stream); break;
     default: return fail(INV_ERR_INVALID_ARG, "inv_obs_from_packed: unknown obs_dtype");
     }
     CUDA_TRY(ce);
@@ -1118,7 +1160,7 @@ int inv_debug_phase(inv_sim *s, int phase, int pid, int arg, int arg2, void *str
     DeviceGuard g(s->cfg.device);
     Params p = base_params(s);
     p.phase = phase; p.pid = pid; p.arg = arg; p.arg2 = arg2;
-    CUDA_TRY((launch_one<OP_DEBUG, INV_OBS_F32, false, false, 32>(p, s->sm_count, (cudaStream_t)stream)));
+    CUDA_TRY((launch_one<OP_DEBUG, INV_OBS_F32, false, false, 32>(p, (cudaStream_t)stream)));
     note_launch(s, (cudaStream_t)stream);
     return INV_OK;
 }
@@ -1140,14 +1182,15 @@ int64_t inv_launch_count(const inv_sim *s) { return s ? s->launches : 0; }
 int inv_gae(const float *reward_dev, const float *value_dev, const uint8_t *done_dev, const float *last_value_dev,
             double gamma, double lam, int32_t T, int64_t N, float *adv_dev, float *ret_dev, void *stream)
 {
+    const char *who = "inv_gae";
+    if (int rc = inv_host::require_sm100(who)) return rc;
     if (!reward_dev || !value_dev || !done_dev || !adv_dev || !ret_dev || T < 0 || N < 0)
-        return fail(INV_ERR_INVALID_ARG, "inv_gae: bad argument");
+        return inv_host::set_error(INV_ERR_INVALID_ARG, who, "bad argument");
     if (T == 0 || N == 0) return INV_OK;
     const int threads = 128;
     gae_kernel<<<(unsigned)((N + threads - 1) / threads), threads, 0, (cudaStream_t)stream>>>(
         reward_dev, value_dev, done_dev, last_value_dev, (float)gamma, (float)(gamma * lam), T, N, adv_dev, ret_dev);
-    CUDA_TRY(cudaGetLastError());
-    return INV_OK;
+    return inv_host::launch_status(who);
 }
 
 } // extern "C"

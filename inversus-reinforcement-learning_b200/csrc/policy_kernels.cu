@@ -25,6 +25,7 @@
 #include <type_traits>
 
 #include "../../include/inversus_b200.h"
+#include "launch_common.h"
 
 namespace {
 
@@ -709,62 +710,43 @@ __global__ void transpose_cast_kernel(const TS *__restrict__ src, int64_t ld_src
     }
 }
 
-int sm_count_cached()
-{
-    static int n[64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64) return 148;
-    if (n[dev] == 0) {
-        cudaDeviceGetAttribute(&n[dev], cudaDevAttrMultiProcessorCount, dev);
-        if (n[dev] <= 0) n[dev] = 148;
-    }
-    return n[dev];
-}
+constexpr const char *kBadC = "unsupported C: needs C % 8 == 0, D % C == 0 and C / 8 dividing the block size";
+constexpr const char *kBadD = "D must be at most 20480";
 
 } // namespace
 
+// INV_LN_BWD=percta: the pointers, B and D have been checked by inv_ln_relu_bwd
 static int ln_relu_bwd_percta(const void *dy, const void *x, const void *res, const void *cbias, const void *gamma,
                     const void *beta, const float *mean, const float *rstd, int64_t B, int32_t D, int32_t C,
                     void *dx, float *dgamma, float *dbeta, float *dcbias, float *partials, void *stream)
 {
-    if (!dy || !x || !gamma || !beta || !mean || !rstd || !dx || !dgamma || !dbeta || !partials || B <= 0 ||
-        D <= 0 || D % 8)
-        return INV_ERR_INVALID_ARG;
-    if (C <= 0 || C % 8 || D % C || kLnThreads % (C / 8) || C > kLnThreads) return INV_ERR_INVALID_ARG;
+    const char *who = "inv_ln_relu_bwd";
+    if (C <= 0 || C % 8 || D % C || kLnThreads % (C / 8) || C > kLnThreads)
+        return inv_host::set_error(INV_ERR_INVALID_ARG, who, kBadC);
     const int cvecs = C / 8;
     const int nvec = D / 8;
     const int maxv = (nvec + kLnThreads - 1) / kLnThreads;
-    if (maxv > 5) return INV_ERR_INVALID_ARG;
-    const int nsm = sm_count_cached();
+    if (maxv > 5) return inv_host::set_error(INV_ERR_INVALID_ARG, who, kBadD);
+    const int nsm = inv_host::sm_count();
     const unsigned grid = (unsigned)(B < nsm ? B : nsm); // one CTA per SM: 2*D floats of shared memory each
     size_t smem = (size_t)2 * D * sizeof(float);
     if (smem < (size_t)kLnThreads * 8 * sizeof(float)) smem = (size_t)kLnThreads * 8 * sizeof(float);
     cudaStream_t st = (cudaStream_t)stream;
-#define LAUNCH(MV)                                                                                              \
-    if (res) {                                                                                                  \
-        cudaFuncSetAttribute(ln_relu_bwd_kernel<MV, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-        ln_relu_bwd_kernel<MV, true><<<grid, kLnThreads, smem, st>>>((const uint4 *)dy, (const uint4 *)x,       \
-            (const uint4 *)res, (const uint4 *)cbias, cvecs, (const uint4 *)gamma, (const uint4 *)beta, mean,    \
-            rstd, B, nvec, (uint4 *)dx, partials);                                                              \
-    } else {                                                                                                    \
-        cudaFuncSetAttribute(ln_relu_bwd_kernel<MV, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-        ln_relu_bwd_kernel<MV, false><<<grid, kLnThreads, smem, st>>>((const uint4 *)dy, (const uint4 *)x,      \
-            nullptr, (const uint4 *)cbias, cvecs, (const uint4 *)gamma, (const uint4 *)beta, mean, rstd, B,      \
-            nvec, (uint4 *)dx, partials);                                                                       \
-    }
-    switch (maxv) {
-    case 1: LAUNCH(1) break;
-    case 2: LAUNCH(2) break;
-    case 3: LAUNCH(3) break;
-    case 4: LAUNCH(4) break;
-    default: LAUNCH(5) break;
-    }
-#undef LAUNCH
-    if (cudaGetLastError() != cudaSuccess) return INV_ERR_CUDA;
+    using Kern = decltype(&ln_relu_bwd_kernel<1, false>);
+    static const Kern kerns[5][2] = {{ln_relu_bwd_kernel<1, false>, ln_relu_bwd_kernel<1, true>},
+                                     {ln_relu_bwd_kernel<2, false>, ln_relu_bwd_kernel<2, true>},
+                                     {ln_relu_bwd_kernel<3, false>, ln_relu_bwd_kernel<3, true>},
+                                     {ln_relu_bwd_kernel<4, false>, ln_relu_bwd_kernel<4, true>},
+                                     {ln_relu_bwd_kernel<5, false>, ln_relu_bwd_kernel<5, true>}};
+    const Kern kern = kerns[maxv - 1][res != nullptr];
+    if (inv_host::allow_dynamic_smem((const void *)kern, smem) != cudaSuccess) return inv_host::launch_status(who);
+    kern<<<grid, kLnThreads, smem, st>>>((const uint4 *)dy, (const uint4 *)x, (const uint4 *)res, (const uint4 *)cbias,
+                                        cvecs, (const uint4 *)gamma, (const uint4 *)beta, mean, rstd, B, nvec, (uint4 *)dx,
+                                        partials);
+    if (int rc = inv_host::launch_status(who)) return rc;
     const int width = 2 * D + C;
     reduce_partials_kernel<<<(width + 255) / 256, 256, 0, st>>>(partials, (int)grid, width, dgamma, dbeta, dcbias, D);
-    return cudaGetLastError() == cudaSuccess ? INV_OK : INV_ERR_CUDA;
+    return inv_host::launch_status(who);
 }
 
 
@@ -773,8 +755,11 @@ extern "C" {
 int inv_transpose_cast(const void *src, int32_t src_is_f32, int64_t ld_src, void *dst, int32_t dst_is_f32,
                        int64_t ld_dst, int64_t rows, int32_t A, int32_t B, void *stream)
 {
-    if (!src || !dst || rows < 0 || A <= 0 || B <= 0 || rows > 65535 || src_is_f32 == dst_is_f32)
-        return INV_ERR_INVALID_ARG;
+    const char *who = "inv_transpose_cast";
+    if (int rc = inv_host::require_sm100(who)) return rc;
+    if (!src || !dst || rows < 0 || A <= 0 || B <= 0 || rows > 65535)
+        return inv_host::set_error(INV_ERR_INVALID_ARG, who, "null pointer, or rows outside [0, 65535], or A or B not positive");
+    if (src_is_f32 == dst_is_f32) return inv_host::set_error(INV_ERR_INVALID_ARG, who, "exactly one side must be fp32");
     if (rows == 0) return INV_OK;
     const dim3 grid((B + 31) / 32, (A + 31) / 32, (unsigned)rows), block(32, 8);
     cudaStream_t st = (cudaStream_t)stream;
@@ -784,22 +769,25 @@ int inv_transpose_cast(const void *src, int32_t src_is_f32, int64_t ld_src, void
     else
         transpose_cast_kernel<__nv_bfloat16, float><<<grid, block, 0, st>>>(
             (const __nv_bfloat16 *)src, ld_src, (float *)dst, ld_dst, A, B);
-    return cudaGetLastError() == cudaSuccess ? INV_OK : INV_ERR_CUDA;
+    return inv_host::launch_status(who);
 }
 
-int inv_ln_relu_partials(int32_t D) { (void)D; return 2 * sm_count_cached(); }
+int inv_ln_relu_partials(int32_t D) { (void)D; return 2 * inv_host::sm_count(); }
 
 int inv_ln_relu_fwd(const void *x, const void *res, const void *cbias, const void *gamma, const void *beta,
                     int64_t B, int32_t D, int32_t C, float eps, void *y, float *mean, float *rstd, void *stream)
 {
-    if (!x || !gamma || !beta || !y || !mean || !rstd || B < 0 || D <= 0 || D % 8) return INV_ERR_INVALID_ARG;
-    if (C <= 0 || C % 8 || D % C || kLnThreads % (C / 8)) return INV_ERR_INVALID_ARG;
+    const char *who = "inv_ln_relu_fwd";
+    if (int rc = inv_host::require_sm100(who)) return rc;
+    if (!x || !gamma || !beta || !y || !mean || !rstd || B < 0 || D <= 0 || D % 8)
+        return inv_host::set_error(INV_ERR_INVALID_ARG, who, "null pointer, B < 0, or D not a positive multiple of 8");
+    if (C <= 0 || C % 8 || D % C || kLnThreads % (C / 8)) return inv_host::set_error(INV_ERR_INVALID_ARG, who, kBadC);
     const int cvecs = C / 8;
     if (B == 0) return INV_OK;
     const int nvec = D / 8;
     const int maxv = (nvec + kLnThreads - 1) / kLnThreads;
-    if (maxv > 5) return INV_ERR_INVALID_ARG; // D <= 20480
-    const int64_t cap = (int64_t)sm_count_cached() * 4;
+    if (maxv > 5) return inv_host::set_error(INV_ERR_INVALID_ARG, who, kBadD);
+    const int64_t cap = (int64_t)inv_host::sm_count() * 4;
     const unsigned grid = (unsigned)(B < cap ? B : cap);
     cudaStream_t st = (cudaStream_t)stream;
 #define LAUNCH(MV)                                                                                              \
@@ -819,16 +807,18 @@ int inv_ln_relu_fwd(const void *x, const void *res, const void *cbias, const voi
     default: LAUNCH(5) break;
     }
 #undef LAUNCH
-    return cudaGetLastError() == cudaSuccess ? INV_OK : INV_ERR_CUDA;
+    return inv_host::launch_status(who);
 }
 
 int inv_ln_relu_bwd(const void *dy, const void *x, const void *res, const void *cbias, const void *gamma,
                     const void *beta, const float *mean, const float *rstd, int64_t B, int32_t D, int32_t C,
                     void *dx, float *dgamma, float *dbeta, float *dcbias, float *partials, void *stream)
 {
+    const char *who = "inv_ln_relu_bwd";
+    if (int rc = inv_host::require_sm100(who)) return rc;
     if (!dy || !x || !gamma || !beta || !mean || !rstd || !dx || !dgamma || !dbeta || !partials || B <= 0 ||
         D <= 0 || D % 8)
-        return INV_ERR_INVALID_ARG;
+        return inv_host::set_error(INV_ERR_INVALID_ARG, who, "null pointer, B <= 0, or D not a positive multiple of 8");
     {   // default: the cluster-split kernel; INV_LN_BWD=percta selects the round-1 kernel (one CTA per
         // SM, shared-memory accumulators) for A/B measurements
         static int use_cluster = -1;
@@ -840,11 +830,12 @@ int inv_ln_relu_bwd(const void *dy, const void *x, const void *res, const void *
             return ln_relu_bwd_percta(dy, x, res, cbias, gamma, beta, mean, rstd, B, D, C, dx, dgamma, dbeta, dcbias,
                                       partials, stream);
     }
-    if (C <= 0 || C % 8 || D % C || kBwdThreads % (C / 8) || C > kBwdThreads) return INV_ERR_INVALID_ARG;
+    if (C <= 0 || C % 8 || D % C || kBwdThreads % (C / 8) || C > kBwdThreads)
+        return inv_host::set_error(INV_ERR_INVALID_ARG, who, kBadC);
     const int cvecs = C / 8;
     const int nvec = D / 8;
     const int cs = (nvec + kBwdThreads - 1) / kBwdThreads; // CTAs per cluster: 2 / 4 / 8 for D = 4800 / 9600 / 19200
-    if (cs > kMaxCluster) return INV_ERR_INVALID_ARG;      // D <= 20480
+    if (cs > kMaxCluster) return inv_host::set_error(INV_ERR_INVALID_ARG, who, kBadD);
     cudaStream_t st = (cudaStream_t)stream;
     // samples per cluster exchange: 4 without a residual input (INV_LN_BWD_S=2 selects 2, for A/B runs), 2 with
     static int s_nores = -1;
@@ -863,7 +854,7 @@ int inv_ln_relu_bwd(const void *dy, const void *x, const void *res, const void *
     attr[0].val.clusterDim.y = 1;
     attr[0].val.clusterDim.z = 1;
     const size_t smem = res ? bwd_cluster_smem<2, true>() : (S == 4 ? bwd_cluster_smem<4, false>() : bwd_cluster_smem<2, false>());
-    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return INV_ERR_CUDA;
+    if (inv_host::allow_dynamic_smem((const void *)kern, smem) != cudaSuccess) return inv_host::launch_status(who);
     cfg.blockDim = dim3(kBwdThreads, 1, 1);
     cfg.dynamicSmemBytes = smem;
     cfg.stream = st;
@@ -880,9 +871,9 @@ int inv_ln_relu_bwd(const void *dy, const void *x, const void *res, const void *
         cfg.gridDim = dim3((unsigned)(cs * 64), 1, 1);
         if (cudaOccupancyMaxActiveClusters(&ncl, kern, &cfg) != cudaSuccess || ncl <= 0) {
             cudaGetLastError();
-            ncl = sm_count_cached() / cs; // conservative: one CTA per SM
+            ncl = inv_host::sm_count() / cs; // conservative: one CTA per SM
         }
-        const int cap = 2 * sm_count_cached() / cs; // the partials buffer holds 2 * SMs parts
+        const int cap = 2 * inv_host::sm_count() / cs; // the partials buffer holds 2 * SMs parts
         if (ncl > cap) ncl = cap;
         if (dev >= 0 && dev < 64) resident[dev][cs][variant] = ncl;
     }
@@ -894,10 +885,10 @@ int inv_ln_relu_bwd(const void *dy, const void *x, const void *res, const void *
     const uint4 *g4 = (const uint4 *)gamma, *b4 = (const uint4 *)beta;
     uint4 *dx4 = (uint4 *)dx;
     if (cudaLaunchKernelEx(&cfg, kern, dy4, x4, res4, cb4, cvecs, g4, b4, mean, rstd, B, nvec, dx4, partials) != cudaSuccess)
-        return INV_ERR_CUDA;
+        return inv_host::launch_status(who);
     const int width = 2 * D + C;
     reduce_cluster_partials_kernel<<<(width + 255) / 256, 256, 0, st>>>(partials, ncl, ncl * cs, D, C, dgamma, dbeta, dcbias);
-    return cudaGetLastError() == cudaSuccess ? INV_OK : INV_ERR_CUDA;
+    return inv_host::launch_status(who);
 }
 
 } // extern "C"

@@ -30,6 +30,7 @@
 #include <stdlib.h>
 
 #include "../../include/inversus_b200.h"
+#include "launch_common.h"
 
 namespace {
 
@@ -297,44 +298,27 @@ bool make_map(CUtensorMap *map, const void *ptr, int64_t B, int C, int box_rows)
                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-int sm_count_wg()
-{
-    static int n[64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64) return 148;
-    if (n[dev] == 0) {
-        cudaDeviceGetAttribute(&n[dev], cudaDevAttrMultiProcessorCount, dev);
-        if (n[dev] <= 0) n[dev] = 148;
-    }
-    return n[dev];
-}
-
 template <int COUT, int CIN, int NKX>
 int launch_wgrad(const void *dy, const void *x, int64_t B, float *dw, float *partials, cudaStream_t st)
 {
+    const char *who = "inv_conv3x3_wgrad";
     typedef Shape<COUT, CIN, NKX> S;
     CUtensorMap map_dy, map_x;
-    if (!make_map(&map_dy, dy, B, COUT, 10) || !make_map(&map_x, x, B, CIN, 12)) return INV_ERR_CUDA;
+    if (!make_map(&map_dy, dy, B, COUT, 10) || !make_map(&map_x, x, B, CIN, 12))
+        return inv_host::set_error(INV_ERR_CUDA, who, "cuTensorMapEncodeTiled failed");
     constexpr size_t smem = (size_t)S::kStages * S::kStageBytes + 1024;
     auto kern = conv3x3_wgrad_kernel<COUT, CIN, NKX>;
-    static bool configured[64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !configured[dev]) {
-        if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return INV_ERR_CUDA;
-        if (dev >= 0 && dev < 64) configured[dev] = true;
-    }
+    if (inv_host::allow_dynamic_smem((const void *)kern, smem) != cudaSuccess) return inv_host::launch_status(who);
     constexpr int KXG = 3 / NKX;
-    int parts = sm_count_wg() / KXG;
+    int parts = inv_host::sm_count() / KXG;
     if (parts > B) parts = (int)B;
     if (parts < 1) parts = 1;
     const int per_part = (int)((B + parts - 1) / parts);
     kern<<<KXG * parts, kThreads, smem, st>>>(map_dy, map_x, B, per_part, partials);
-    if (cudaGetLastError() != cudaSuccess) return INV_ERR_CUDA;
+    if (int rc = inv_host::launch_status(who)) return rc;
     const int total = 9 * COUT * CIN;
     wgrad_reduce_kernel<<<(total + 255) / 256, 256, 0, st>>>(partials, parts, CIN, COUT, dw);
-    return cudaGetLastError() == cudaSuccess ? INV_OK : INV_ERR_CUDA;
+    return inv_host::launch_status(who);
 }
 
 } // namespace
@@ -344,19 +328,22 @@ extern "C" {
 int64_t inv_conv3x3_wgrad_scratch_floats(int32_t cin, int32_t cout)
 {
     const int kxg = cin == 128 ? 3 : 1; // conv4: three CTAs per sample range; conv2 / conv3: up to one part per SM
-    return (int64_t)(sm_count_wg() / kxg) * 9 * cout * cin;
+    return (int64_t)(inv_host::sm_count() / kxg) * 9 * cout * cin;
 }
 
 int inv_conv3x3_wgrad(const void *dy, const void *x, int64_t B, int32_t cin, int32_t cout, float *dw, float *partials,
                       void *stream)
 {
-    if (!dy || !x || !dw || !partials || B <= 0) return INV_ERR_INVALID_ARG;
-    if (((uintptr_t)dy | (uintptr_t)x) & 15u) return INV_ERR_INVALID_ARG;
+    const char *who = "inv_conv3x3_wgrad";
+    if (int rc = inv_host::require_sm100(who)) return rc;
+    if (!dy || !x || !dw || !partials || B <= 0) return inv_host::set_error(INV_ERR_INVALID_ARG, who, "null pointer or B <= 0");
+    if (((uintptr_t)dy | (uintptr_t)x) & 15u)
+        return inv_host::set_error(INV_ERR_INVALID_ARG, who, "dy and x must be 16-byte aligned");
     cudaStream_t st = (cudaStream_t)stream;
     if (cout == 128 && cin == 128) return launch_wgrad<128, 128, 1>(dy, x, B, dw, partials, st);
     if (cout == 128 && cin == 64) return launch_wgrad<128, 64, 1>(dy, x, B, dw, partials, st);
     if (cout == 64 && cin == 32) return launch_wgrad<64, 32, 3>(dy, x, B, dw, partials, st);
-    return INV_ERR_INVALID_ARG;
+    return inv_host::set_error(INV_ERR_INVALID_ARG, who, "(cout, cin) must be (128, 128), (128, 64) or (64, 32)");
 }
 
 } // extern "C"
