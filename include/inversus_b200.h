@@ -49,6 +49,9 @@ extern "C" {
 #define INV_TABLE_STRIDE 64
 #define INV_TABLE_RESET_OFF 16
 #define INV_STREAM_RESET 0xFFFFFFFFu
+/* the third counter word of seat 0's draws in inv_scripted_actions is INV_STREAM_SEAT0 | step_count
+ * (step_count < 2^31): a range no simulator stream (step_count, INV_STREAM_RESET) can reach */
+#define INV_STREAM_SEAT0 0x80000000u
 
 typedef enum {
     INV_OK = 0,
@@ -337,6 +340,23 @@ int inv_episode_tally(const uint8_t *done, const uint8_t *info, const int32_t *e
                       const double *episode_return, const void *packed_dev, int64_t stride, int64_t count, int64_t quota,
                       int32_t max_episode_steps, int32_t *counts_dev, double *return_sum_dev, int32_t *remaining_dev,
                       void *stream);
+
+/* inv_scripted_actions: the scripted dummy (env_wrappers.py:69-170) as a player of either seat, one
+ *   int8 action id per env into actions_out [count], from the pre-step packed state (planes 0-2 of
+ *   entries [0, count); csrc/eval_kernels.cu, DESIGN.md "evaluator"). Handle-free, one launch on
+ *   `stream`, capturable in a CUDA graph, no synchronisation. difficulty: INV_DIFFICULTY_EASY / _HARD.
+ *   seat 1 (P2): exactly the opponent of an INV_MODE_DUMMY step, drawing from counter
+ *     (gid_base + i, episode, step_count, k/4), the stream that step consumes. A selfplay handle
+ *     stepped with a_p2 = these ids reproduces a dummy-mode handle of the same seed, env ids and P1
+ *     actions bit for bit.
+ *   seat 0 (P1): the same rule with the roles exchanged: it chases / shoots at P2, steps only onto
+ *     WHITE (P1's walkable colour) and returns 0 without a draw when P1 is dead; counter
+ *     (gid_base + i, episode, INV_STREAM_SEAT0 | step_count, k/4).
+ *   The fourth counter word k/4 < 16 keeps both apart from inv_select_actions (0x80000000 | seat).
+ *   INV_ERR_INVALID_ARG: count < 0, NULL pointers, stride < count, seat or difficulty not 0/1,
+ *   gid_base outside [0, 2^32 - count]. */
+int inv_scripted_actions(const void *packed_dev, int64_t stride, int64_t count, int64_t gid_base, uint64_t seed,
+                         int seat, int difficulty, int8_t *actions_out, void *stream);
 
 /* kernel launches issued through this handle so far (bench.py's gpu_launches) */
 int64_t inv_launch_count(const inv_sim *sim);

@@ -94,6 +94,8 @@ SYMBOLS = {
     "inv_select_actions": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_uint64, C.c_int,
                                      C.c_int, C.c_void_p, C.c_void_p]),
     "inv_episode_tally": (C.c_int, [C.c_void_p] * 5 + [C.c_int64, C.c_int64, C.c_int64, C.c_int32] + [C.c_void_p] * 4),
+    "inv_scripted_actions": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_uint64, C.c_int, C.c_int,
+                                       C.c_void_p, C.c_void_p]),
 }
 
 _lib = None

@@ -8,8 +8,10 @@
 //   inv_episode_tally   per-env wins / losses / draws / length sum / return sum of exactly the
 //                       first `quota` episodes of every env, plus the number of envs still short
 //                       of their quota.
+//   inv_scripted_actions the scripted dummy as a player of either seat: one int8 action id per
+//                       env, drawn from counters that are a pure function of the simulator state.
 //
-// Both read the counter words through the packed-state codec (load_counters). Every value has one
+// They read the packed state through its codec (load_counters, load_board). Every value has one
 // owner thread; the only atomic adds an integer count into `remaining`, whose sum does not depend
 // on the order of the additions.
 #include "inversus_kernels.cuh"
@@ -22,6 +24,7 @@ namespace {
 constexpr int kA = INV_NUM_ACTIONS;
 constexpr int kSelThreads = 256;
 constexpr int kTallyThreads = 256;
+constexpr int kScriptThreads = 256;
 
 // One thread per row. The block's rows are staged through shared memory so that the global reads
 // are coalesced; a row's 13 floats then sit at an odd word stride, which is bank-conflict free.
@@ -105,6 +108,21 @@ episode_tally_kernel(const uint8_t *__restrict__ done, const uint8_t *__restrict
     if (threadIdx.x == 0 && n) atomicAdd(remaining, n);
 }
 
+// One thread per env: planes 0-2 in (48 B), one action id out.
+__global__ void __launch_bounds__(kScriptThreads)
+scripted_actions_kernel(const uint4 *__restrict__ packed, int64_t stride, int64_t count, uint32_t gid_base,
+                        uint32_t seed_lo, uint32_t seed_hi, int seat, int difficulty, int8_t *__restrict__ out)
+{
+    const int64_t i = (int64_t)blockIdx.x * kScriptThreads + threadIdx.x;
+    if (i >= count) return;
+    Env s;
+    load_board(s, packed, stride, i);
+    Params p; // Draws reads only the key from it
+    p.seed_lo = seed_lo;
+    p.seed_hi = seed_hi;
+    out[i] = (int8_t)scripted_action(s, p, gid_base + (uint32_t)i, seat, difficulty);
+}
+
 } // namespace
 
 extern "C" {
@@ -145,6 +163,22 @@ int inv_episode_tally(const uint8_t *done, const uint8_t *info, const int32_t *e
     episode_tally_kernel<<<(unsigned)blocks, kTallyThreads, 0, st>>>(
         done, info, episode_steps, episode_return, static_cast<const uint4 *>(packed_dev), stride, count,
         (uint32_t)quota, counts_dev, return_sum_dev, remaining_dev);
+    return inv_host::launch_status(who);
+}
+
+int inv_scripted_actions(const void *packed_dev, int64_t stride, int64_t count, int64_t gid_base, uint64_t seed,
+                         int seat, int difficulty, int8_t *actions_out, void *stream)
+{
+    const char *who = "inv_scripted_actions";
+    if (int rc = inv_host::require_sm100(who)) return rc;
+    if (count < 0 || !packed_dev || !actions_out || stride < count || (seat != 0 && seat != 1) ||
+        (difficulty != 0 && difficulty != 1) || gid_base < 0 || gid_base > 0x100000000ll - count)
+        return inv_host::set_error(INV_ERR_INVALID_ARG, who, "bad argument");
+    if (count == 0) return INV_OK;
+    const int64_t blocks = (count + kScriptThreads - 1) / kScriptThreads;
+    scripted_actions_kernel<<<(unsigned)blocks, kScriptThreads, 0, (cudaStream_t)stream>>>(
+        static_cast<const uint4 *>(packed_dev), stride, count, (uint32_t)gid_base, (uint32_t)seed,
+        (uint32_t)(seed >> 32), seat, difficulty, actions_out);
     return inv_host::launch_status(who);
 }
 

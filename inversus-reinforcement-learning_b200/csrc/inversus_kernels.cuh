@@ -213,11 +213,9 @@ INV_HD Counters load_counters(const uint4 *st, int64_t stride, int64_t i)
     return counters_from_planes(st[stride + i], st[2 * stride + i]);
 }
 
-template <int E>
-INV_HD void load_env(Env &s, uint16_t *sb, const uint4 *st, int64_t stride, int64_t i)
+// Everything but the bullet column, from planes 0-2.
+INV_HD void board_from_planes(Env &s, const uint4 &a, const uint4 &b, const uint4 &c)
 {
-    const uint4 a = st[i], b = st[stride + i], c = st[2 * stride + i];
-    const uint4 d = st[3 * stride + i], e = st[4 * stride + i];
     s.t[0] = a.x; s.t[1] = a.y; s.t[2] = a.z; s.t[3] = a.w; s.t[4] = b.x;
     unpack_player(s, 0, b.y);
     s.nb = (int)(b.y >> 20) & 31;
@@ -226,6 +224,20 @@ INV_HD void load_env(Env &s, uint16_t *sb, const uint4 *st, int64_t stride, int6
     s.step = k.step;
     s.episode = k.episode;
     s.ret = double_from_words(c.y, c.z);
+}
+// Planes 0-2 only (48 of the 80 bytes): tiles, players and counters, for consumers that never
+// read a bullet (the scripted players of inv_scripted_actions).
+INV_HD void load_board(Env &s, const uint4 *st, int64_t stride, int64_t i)
+{
+    board_from_planes(s, st[i], st[stride + i], st[2 * stride + i]);
+}
+
+template <int E>
+INV_HD void load_env(Env &s, uint16_t *sb, const uint4 *st, int64_t stride, int64_t i)
+{
+    const uint4 a = st[i], b = st[stride + i], c = st[2 * stride + i];
+    const uint4 d = st[3 * stride + i], e = st[4 * stride + i];
+    board_from_planes(s, a, b, c);
     const uint32_t w[8] = {d.x, d.y, d.z, d.w, e.x, e.y, e.z, e.w};
 #pragma unroll
     for (int k = 0; k < 8; ++k) {
@@ -500,10 +512,13 @@ __device__ __forceinline__ void engine_reset(Env &s, Draws &dr)
 
 // ---- wrapper: env_wrappers.py ----
 
-__device__ __forceinline__ bool p2_can_step(const Env &s, int dir) // env_wrappers.py:115-119
+// env_wrappers.py:115-119 for the player P: on the board and on the colour try_move lets P enter
+// (WHITE for P1, BLACK for P2)
+template <int P>
+__device__ __forceinline__ bool can_step(const Env &s, int dir)
 {
-    const int nx = s.x[1] + dir_dx(dir), ny = s.y[1] + dir_dy(dir);
-    return in_bounds(nx, ny) && tile_white(s, nx, ny) == 0u;
+    const int nx = s.x[P] + dir_dx(dir), ny = s.y[P] + dir_dy(dir);
+    return in_bounds(nx, ny) && tile_white(s, nx, ny) == (uint32_t)(P == 0);
 }
 
 // four 2-bit direction fields; random.shuffle = Fisher-Yates from the top (CPython Lib/random.py)
@@ -519,42 +534,60 @@ __device__ __forceinline__ uint32_t shuffle4(uint32_t d, Draws &dr)
     return d;
 }
 
-// env_wrappers.py:69-170. Returns P2's action id; consumes 0..9 draws in the reference's order.
+// env_wrappers.py:69-170 played by player P against player 1 - P. Returns P's action id; consumes
+// 0..9 draws in the reference's order. P = 1 is the reference's dummy (the simulator's opponent);
+// P = 0 is the same rule with the roles exchanged (inv_scripted_actions, seat 0).
+template <int P>
 __device__ __forceinline__ int dummy_policy(const Env &s, Draws &dr, int difficulty)
 {
-    if (!s.alive[1]) return 0; // :77-78, no draw
+    constexpr int Q = 1 - P; // the player chased
+    if (!s.alive[P]) return 0; // :77-78, no draw
     const bool hard = difficulty != 0;
-    const bool x_al = s.x[1] == s.x[0], y_al = s.y[1] == s.y[0];
+    const bool x_al = s.x[P] == s.x[Q], y_al = s.y[P] == s.y[Q];
     const bool should_shoot = dr.next() < (hard ? kThreshShootHard : 0u); // :96
-    if (should_shoot && s.ammo[1] > 0 && (x_al || y_al)) {
-        if (x_al) return 5 + (s.y[0] < s.y[1] ? 0 : 2);  // :98-99 UP / DOWN (DOWN on the same tile)
-        return 5 + (s.x[0] < s.x[1] ? 3 : 1);            // :100-101 LEFT / RIGHT
+    if (should_shoot && s.ammo[P] > 0 && (x_al || y_al)) {
+        if (x_al) return 5 + (s.y[Q] < s.y[P] ? 0 : 2);  // :98-99 UP / DOWN (DOWN on the same tile)
+        return 5 + (s.x[Q] < s.x[P] ? 3 : 1);            // :100-101 LEFT / RIGHT
     }
     uint32_t dirs = 0u | (2u << 2) | (3u << 4) | (1u << 6); // [UP, DOWN, LEFT, RIGHT]  :104
     if (dr.next() < (hard ? kThreshRandMoveHard : 0u)) {    // :105
         dirs = shuffle4(dirs, dr);
         const int c = dirs & 3u;
-        if (p2_can_step(s, c)) return 1 + c;
+        if (can_step<P>(s, c)) return 1 + c;
     }
     if (!hard) {                                            // :122-124
         if (!(dr.next() < kThreshMoveEasy)) return 0;
     }
-    const int dx = s.x[0] - s.x[1], dy = s.y[0] - s.y[1];   // :127-136
+    const int dx = s.x[Q] - s.x[P], dy = s.y[Q] - s.y[P];   // :127-136
     int c0 = -1, c1 = -1;
     if (dx != 0) c0 = dx > 0 ? 1 : 3;
     if (dy != 0) { const int v = dy > 0 ? 2 : 0; if (c0 < 0) c0 = v; else c1 = v; }
     if (c1 >= 0) { // shuffle of a 2-list: j = randbelow(2); swap(x[1], x[j])   :138
         if (dr.below(2) == 0) { const int t = c0; c0 = c1; c1 = t; }
     }
-    if (c0 >= 0 && p2_can_step(s, c0)) return 1 + c0;
-    if (c1 >= 0 && p2_can_step(s, c1)) return 1 + c1;
+    if (c0 >= 0 && can_step<P>(s, c0)) return 1 + c0;
+    if (c1 >= 0 && can_step<P>(s, c1)) return 1 + c1;
     dirs = shuffle4(dirs, dr);                              // :155 (possibly already permuted)
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
         const int c = (dirs >> (2 * i)) & 3u;
-        if (p2_can_step(s, c)) return 1 + c;
+        if (can_step<P>(s, c)) return 1 + c;
     }
     return 0;
+}
+
+// The third counter word of the scripted draws of inv_scripted_actions for `seat`: the step's
+// opponent stream (seat 1, what a dummy-mode step consumes) or 0x80000000 | step_count (seat 0),
+// which no simulator stream (step_count < 2^31, INV_STREAM_RESET) can equal.
+INV_HD uint32_t scripted_stream(int seat, uint32_t step) { return seat ? step : (INV_STREAM_SEAT0 | step); }
+
+// inv_scripted_actions for one env: the scripted rule played by `seat` (0 = P1, 1 = P2) on the
+// pre-step state, with the draws of counter (gid, episode, scripted_stream(seat, step_count), k/4).
+__device__ __forceinline__ int scripted_action(const Env &s, const Params &p, uint32_t gid, int seat, int difficulty)
+{
+    Draws dr;
+    dr.init(p, gid, s.episode, scripted_stream(seat, s.step), nullptr);
+    return seat ? dummy_policy<1>(s, dr, difficulty) : dummy_policy<0>(s, dr, difficulty);
 }
 
 // (float)(k / 6.0) for the extra vector (env_wrappers.py:238-243)
@@ -626,7 +659,7 @@ __device__ __forceinline__ StepResult rl_step(Env &s, uint16_t *sb, int a1, int 
     if (p.mode == INV_MODE_DUMMY) { // env_wrappers.py:305-306
         Draws dr;
         dr.init(p, gid, s.episode, s.step, trow);
-        a2 = dummy_policy(s, dr, p.difficulty);
+        a2 = dummy_policy<1>(s, dr, p.difficulty);
     } else if ((unsigned)a2 > 12u) { // :307-314, the caller ran opponent_policy
         atomicOr(p.status, INV_STATUS_INVALID_ACTION);
         a2 = 0;
@@ -711,7 +744,7 @@ __device__ __forceinline__ uint8_t debug_phase(Env &s, uint16_t *sb, const Param
     case INV_PHASE_DUMMY_POLICY: {
         Draws dr;
         dr.init(p, gid, s.episode, s.step, trow);
-        res = dummy_policy(s, dr, p.difficulty);
+        res = dummy_policy<1>(s, dr, p.difficulty);
         break;
     }
     default: break;

@@ -8,6 +8,7 @@ K episodes of every env, so short episodes are not over-represented. The host re
 every 32 steps; nothing else leaves the GPU until the end (DESIGN.md "evaluator").
 
     python -m inversus_b200.evaluate --model A.pt --opponent hard --num_envs 65536 --episodes_per_env 4
+    python -m inversus_b200.evaluate --model A.pt --opponent hard --seats both ...   # the dummy in either seat
     torchrun --nproc-per-node 8 -m inversus_b200.evaluate --model A.pt --opponent B.pt --num_envs 1048576 ...
 """
 from __future__ import annotations
@@ -31,6 +32,7 @@ from .simulator import BatchedInversus
 
 SCRIPTED = ("easy", "hard")
 ACTIONS = ("greedy", "sample")
+SEATS = ("p1", "both")
 CHECK_EVERY = 32  # steps between the host's reads of the `remaining` counter
 Z95 = NormalDist().inv_cdf(0.975)
 
@@ -96,6 +98,47 @@ def select_actions(logits: torch.Tensor, ps: PackedStates, *, seed: int, seat: i
     return out
 
 
+def scripted_actions(ps: PackedStates, *, seat: int, difficulty, seed: int, gid_base: int = 0,
+                     out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """int8 action ids of the scripted dummy playing `seat` (0 = P1, 1 = P2) on the envs of `ps`
+    (entry i = env gid_base + i), from their pre-step packed states (inv_scripted_actions). Seat 1
+    is exactly the opponent of a dummy-mode step. difficulty: "easy" / "hard" (or 0 / 1)."""
+    difficulty = _capi.DIFFICULTY[difficulty] if isinstance(difficulty, str) else int(difficulty)
+    dev = ps.planes.device
+    n = len(ps)
+    if out is None:
+        out = torch.empty(n, dtype=torch.int8, device=dev)
+    assert out.dtype == torch.int8 and out.is_contiguous() and out.numel() == n
+    ptr, stride, count = _packed_args(ps)
+    with torch.cuda.device(dev):
+        _capi.check(_capi.load().inv_scripted_actions(ptr, stride, count, int(gid_base), int(seed) & 0xFFFFFFFFFFFFFFFF,
+                                                      int(seat), difficulty, out.data_ptr(), _stream(dev)))
+    return out
+
+
+def seat_actions(view: PackedStates, segments, *, seat: int, seed: int, gid_base: int, out: torch.Tensor,
+                 logits: Optional[torch.Tensor] = None, greedy: bool = True, act_chunk: int = 65536) -> torch.Tensor:
+    """Seat `seat`'s int8 action ids for all envs of `view` (entry i = env gid_base + i), built
+    segment by segment into `out`. `segments` lists (player, lo, hi) over [0, len(view)): a player is
+    "easy" / "hard" (the scripted dummy, inv_scripted_actions) or a `PackedStates -> logits`
+    callable, run in micro-batches of `act_chunk` into the fp32 `logits` buffer [len(view), 13] and
+    turned into ids by inv_select_actions (greedy or sampled)."""
+    with torch.no_grad():
+        for player, lo, hi in segments:
+            if lo >= hi:
+                continue
+            if isinstance(player, str):
+                scripted_actions(view.chunk(lo, hi), seat=seat, difficulty=player, seed=seed, gid_base=gid_base + lo,
+                                 out=out[lo:hi])
+                continue
+            for a in range(lo, hi, act_chunk):
+                b = min(a + act_chunk, hi)
+                logits[a:b].copy_(player(view.chunk(a, b)))
+            select_actions(logits[lo:hi], view.chunk(lo, hi), seed=seed, seat=seat, greedy=greedy,
+                           gid_base=gid_base + lo, out=out[lo:hi])
+    return out
+
+
 def episode_tally(sim: BatchedInversus, quota: int, counts: torch.Tensor, return_sum: torch.Tensor,
                   remaining: torch.Tensor) -> None:
     """Add the episodes that ended in `sim`'s last step into the per-env accumulators
@@ -134,31 +177,39 @@ def _logits_fn(p, device: torch.device) -> Callable[[PackedStates], torch.Tensor
     raise TypeError(f"not a policy: {p!r}")
 
 
-def _check_args(opponent, num_envs: int, episodes_per_env: int, actions: str, max_episode_steps: int) -> bool:
-    """Raises ValueError on a bad combination; returns True for head to head."""
+def _check_args(opponent, num_envs: int, episodes_per_env: int, actions: str, max_episode_steps: int,
+                seats: str = "p1") -> bool:
+    """Raises ValueError on a bad combination; returns True when the policy plays both seats (head
+    to head, or the scripted dummy with seats="both")."""
     if actions not in ACTIONS:
         raise ValueError(f"actions must be one of {ACTIONS}, got {actions!r}")
+    if seats not in SEATS:
+        raise ValueError(f"seats must be one of {SEATS}, got {seats!r}")
     if isinstance(opponent, str) and opponent not in SCRIPTED and not os.path.isfile(opponent):
         raise ValueError(f"opponent must be 'easy', 'hard', a policy or a checkpoint file, got {opponent!r}")
     head_to_head = not (isinstance(opponent, str) and opponent in SCRIPTED)
+    two_seats = head_to_head or seats == "both"
     if episodes_per_env < 1:
         raise ValueError("episodes_per_env must be at least 1")
-    if num_envs < (2 if head_to_head else 1):
+    if num_envs < (2 if two_seats else 1):
         raise ValueError("head to head needs at least 2 envs (one per seat)" if head_to_head
+                         else "seats='both' needs at least 2 envs (one per seat)" if two_seats
                          else "num_envs must be at least 1")
     if max_episode_steps < 1 or episodes_per_env * max_episode_steps >= 1 << 31:
         raise ValueError("episodes_per_env * max_episode_steps must be below 2^31")
-    return head_to_head
+    return two_seats
 
 
 def play_shard(policy, opponent, num_envs: int, episodes_per_env: int, first: int, count: int, *,
                actions: str = "greedy", seed: int, max_episode_steps: int = 500, act_chunk: Optional[int] = None,
-               cuda_graph: Optional[bool] = None, device=None) -> dict:
+               cuda_graph: Optional[bool] = None, device=None, seats: str = "p1") -> dict:
     """Play the envs with global ids [first, first + count) of an evaluation over `num_envs` envs
     (what one rank does) and return their raw tallies from the policy's side:
     `seats` int64 [2, 4] (rows: policy as P1, policy as P2; columns: wins, losses, draws, length
-    sum), `p1_return_sum` (P1's summed episode return over the shard), `env_steps` and `steps`."""
-    head_to_head = _check_args(opponent, num_envs, episodes_per_env, actions, max_episode_steps)
+    sum), `p1_return_sum` (P1's summed episode return over the shard's policy-as-P1 envs),
+    `env_steps` and `steps`."""
+    two_seats = _check_args(opponent, num_envs, episodes_per_env, actions, max_episode_steps, seats)
+    head_to_head = not (isinstance(opponent, str) and opponent in SCRIPTED)
     if not (0 <= first and 1 <= count and first + count <= num_envs):
         raise ValueError("the shard must lie inside [0, num_envs)")
     dev = torch.device("cuda", torch.cuda.current_device() if device is None else torch.device(device).index or 0)
@@ -166,12 +217,13 @@ def play_shard(policy, opponent, num_envs: int, episodes_per_env: int, first: in
     ch = int(act_chunk or 65536)
     greedy = actions == "greedy"
     pol = _logits_fn(policy, dev)
-    opp = _logits_fn(opponent, dev) if head_to_head else None
-    sim = BatchedInversus(n, "selfplay" if head_to_head else "dummy", "easy" if head_to_head else opponent,
+    # the scripted dummy of a seats="both" run plays through inv_scripted_actions, not the step
+    opp = _logits_fn(opponent, dev) if head_to_head else opponent
+    sim = BatchedInversus(n, "selfplay" if two_seats else "dummy", "easy" if two_seats else opponent,
                           max_episode_steps, seed=seed, device=dev.index, obs_dtype="none", auto_reset=True,
                           env_id_base=first)
-    # head to head: global ids [0, ceil(N/2)) seat the policy as P1, the rest as P2
-    split = min(max(-(-num_envs // 2) - first, 0), n) if head_to_head else n
+    # both seats: global ids [0, ceil(N/2)) seat the policy as P1, the rest as P2
+    split = min(max(-(-num_envs // 2) - first, 0), n) if two_seats else n
     seats1 = [(pol, 0, split), (opp, split, n)]  # who plays P1 on which local envs
     seats2 = [(opp, 0, split), (pol, split, n)]
     with torch.cuda.device(dev):
@@ -183,17 +235,12 @@ def play_shard(policy, opponent, num_envs: int, episodes_per_env: int, first: in
         remaining = torch.zeros(1, dtype=torch.int32, device=dev)
 
         def act(view: int, segments) -> torch.Tensor:
-            with torch.no_grad():
-                for fn, lo, hi in segments:
-                    for a in range(lo, hi, ch):
-                        b = min(a + ch, hi)
-                        logits[view][a:b].copy_(fn(views[view].chunk(a, b)))
-            return select_actions(logits[view], views[view], seed=sim.seed, seat=view, greedy=greedy,
-                                  gid_base=first, out=acts[view])
+            return seat_actions(views[view], segments, seat=view, seed=sim.seed, gid_base=first, out=acts[view],
+                                logits=logits[view], greedy=greedy, act_chunk=ch)
 
         def one_step():
             a1 = act(0, seats1)
-            a2 = act(1, seats2) if head_to_head else None
+            a2 = act(1, seats2) if two_seats else None
             sim.step(a1, a2)
             episode_tally(sim, K, counts, ret, remaining)
 
@@ -236,7 +283,7 @@ def play_shard(policy, opponent, num_envs: int, episodes_per_env: int, first: in
         c = counts.to(torch.int64)
         side1 = c[:, :split].sum(1)                     # policy is P1: P1's wins are its wins
         side2 = c[:, split:].sum(1)[[1, 0, 2, 3]]       # policy is P2: P1's losses are its wins
-        out = {"seats": torch.stack([side1, side2]).cpu(), "p1_return_sum": ret.sum(),
+        out = {"seats": torch.stack([side1, side2]).cpu(), "p1_return_sum": ret[:split].sum(),
                "env_steps": steps * n, "steps": steps}
     del graph
     sim.close()
@@ -244,20 +291,25 @@ def play_shard(policy, opponent, num_envs: int, episodes_per_env: int, first: in
 
 
 def evaluate(policy, opponent, num_envs: int, episodes_per_env: int, *, actions: str = "greedy", seed: int,
-             max_episode_steps: int = 500, act_chunk: Optional[int] = None, cuda_graph: Optional[bool] = None) -> dict:
+             max_episode_steps: int = 500, act_chunk: Optional[int] = None, cuda_graph: Optional[bool] = None,
+             seats: str = "p1") -> dict:
     """Play `policy` for exactly `episodes_per_env` episodes in each of `num_envs` envs (global
     count; under torchrun every rank plays its `shard_range`) against `opponent`: "easy" / "hard"
     (the scripted dummy) or a second policy, head to head with seats split by global env id.
     A policy is an InversusCNNPolicy, a checkpoint path, or a callable PackedStates -> fp32 logits
     [n, 13]. actions: "greedy" (argmax) or "sample" (one counter-based draw per env and step).
-    Returns the result dict; wins / losses / draws are from `policy`'s side."""
-    head_to_head = _check_args(opponent, num_envs, episodes_per_env, actions, max_episode_steps)
+    seats (scripted opponent only): "p1" seats the policy as P1 in every env; "both" splits the
+    seats by global env id as head to head does, the dummy playing the other seat. Returns the
+    result dict; wins / losses / draws are from `policy`'s side."""
+    _check_args(opponent, num_envs, episodes_per_env, actions, max_episode_steps, seats)
+    head_to_head = not (isinstance(opponent, str) and opponent in SCRIPTED)
     rank, local_rank, world = init_distributed()
     dev = torch.device("cuda", local_rank if world > 1 else torch.cuda.current_device())
     first, n_local = shard_range(num_envs, rank, world)
     t0 = time.time()
     raw = play_shard(policy, opponent, num_envs, episodes_per_env, first, n_local, actions=actions, seed=seed,
-                     max_episode_steps=max_episode_steps, act_chunk=act_chunk, cuda_graph=cuda_graph, device=dev)
+                     max_episode_steps=max_episode_steps, act_chunk=act_chunk, cuda_graph=cuda_graph, device=dev,
+                     seats=seats)
     ints = torch.cat([raw["seats"].flatten(), torch.tensor([raw["env_steps"]])]).to(dev)
     rsum = raw["p1_return_sum"].reshape(1).to(dev)
     if world > 1:
@@ -265,19 +317,21 @@ def evaluate(policy, opponent, num_envs: int, episodes_per_env: int, *, actions:
         torch.distributed.all_reduce(rsum)
     ints, rsum = ints.tolist(), float(rsum.item())
     wall = time.time() - t0
-    seats = [ints[0:4], ints[4:8]]
+    per_seat = [ints[0:4], ints[4:8]]
     env_steps = ints[8]
-    tot = [seats[0][k] + seats[1][k] for k in range(4)]
+    tot = [per_seat[0][k] + per_seat[1][k] for k in range(4)]
     res = _rates(*tot)
     assert res["episodes"] == num_envs * episodes_per_env, (res["episodes"], num_envs, episodes_per_env)
-    res["mean_return"] = None if head_to_head else rsum / res["episodes"]
-    res["per_seat"] = {"p1": _rates(*seats[0]), "p2": _rates(*seats[1])}
+    # the shaped reward is P1's: its mean over the policy-as-P1 episodes
+    p1_episodes = sum(per_seat[0][:3])
+    res["mean_return"] = None if head_to_head else rsum / p1_episodes
+    res["per_seat"] = {"p1": _rates(*per_seat[0]), "p2": _rates(*per_seat[1])}
     res.update({"env_steps": env_steps, "wall_s": wall, "env_steps_per_s": env_steps / wall,
                 "episodes_per_s": res["episodes"] / wall})
     res["args"] = {"policy": _describe(policy), "opponent": _describe(opponent), "num_envs": num_envs,
                    "episodes_per_env": episodes_per_env, "actions": actions, "seed": seed,
                    "max_episode_steps": max_episode_steps, "act_chunk": act_chunk or 65536,
-                   "cuda_graph": cuda_graph, "n_gpus": world}
+                   "cuda_graph": cuda_graph, "n_gpus": world, "seats": seats}
     return res
 
 
@@ -293,12 +347,15 @@ def main(argv=None) -> int:
     ap.add_argument("--act_chunk", type=int, default=None, help="samples per inference micro-batch (65536)")
     ap.add_argument("--cuda-graph", choices=["auto", "on", "off"], default="auto",
                     help="replay one captured step (auto: when <= 8192 envs per GPU)")
+    ap.add_argument("--seats", choices=SEATS, default="p1",
+                    help="scripted opponent: the policy plays P1 only, or P1 in the first half of the envs "
+                         "and P2 in the rest (a policy opponent always plays both)")
     ap.add_argument("--json", default=None, help="also write the result to this file")
     a = ap.parse_args(argv)
     if not os.path.isfile(a.model):
         ap.error(f"--model {a.model}: no such file")
     try:
-        _check_args(a.opponent, a.num_envs, a.episodes_per_env, a.actions, a.max_episode_steps)
+        _check_args(a.opponent, a.num_envs, a.episodes_per_env, a.actions, a.max_episode_steps, a.seats)
     except ValueError as e:
         ap.error(str(e))
     if not torch.cuda.is_available():
@@ -306,7 +363,7 @@ def main(argv=None) -> int:
         return 1
     res = evaluate(a.model, a.opponent, a.num_envs, a.episodes_per_env, actions=a.actions, seed=a.seed,
                    max_episode_steps=a.max_episode_steps, act_chunk=a.act_chunk,
-                   cuda_graph={"auto": None, "on": True, "off": False}[a.cuda_graph])
+                   cuda_graph={"auto": None, "on": True, "off": False}[a.cuda_graph], seats=a.seats)
     if int(os.environ.get("RANK", 0)) == 0:
         line = json.dumps(res)
         print(line, flush=True)
