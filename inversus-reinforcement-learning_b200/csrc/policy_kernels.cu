@@ -453,7 +453,7 @@ ln_relu_bwd_cluster_kernel(const uint4 *__restrict__ dy, const uint4 *__restrict
     __shared__ __align__(8) uint64_t s_full[kBwdStages]; // TMA completion per ring stage
     __shared__ __align__(8) uint64_t s_sum[kSumSlots];   // peers' row-sum bytes per group slot
     __shared__ float s_peer[kSumSlots][kMaxCluster][2 * S];
-    __shared__ float s_warp[kBwdThreads / 32][2 * S];
+    __shared__ float s_warp[2][kBwdThreads / 32][2 * S]; // by group parity (see the exchange below)
     __shared__ float s_cb[kBwdThreads * 8];
     __shared__ float s_stat[kBwdStages][2 * S]; // rstd[S], mean[S] of the group in each ring stage
 
@@ -585,7 +585,7 @@ ln_relu_bwd_cluster_kernel(const uint4 *__restrict__ dy, const uint4 *__restrict
             }
 #pragma unroll
             for (; o > 0; o >>= 1) v[0] += __shfl_xor_sync(0xffffffffu, v[0], o);
-            if ((lane & (kRep - 1)) == 0) s_warp[warp][lane / kRep] = v[0];
+            if ((lane & (kRep - 1)) == 0) s_warp[i & 1][warp][lane / kRep] = v[0];
         }
         __syncthreads(); // s_warp is complete, and every thread is done reading ring stage `stage`
         if (tid == 0 && i + kBwdStages < G) issue(i + kBwdStages);
@@ -596,15 +596,20 @@ ln_relu_bwd_cluster_kernel(const uint4 *__restrict__ dy, const uint4 *__restrict
         // This CTA's 2*S sums go to every CTA of the cluster (itself included); the receiver's mbarrier
         // counts the bytes. Two slots are enough: a peer sends group i+1 only after it has passed its
         // wait for group i, and it sends group i+2 only after THIS CTA's sums of i+1 -- sent after all
-        // its warps finished reading slot i -- have reached it. For the same reason s_warp is not
-        // overwritten early: no warp passes the wait below before warp 0 has read s_warp and sent.
+        // its warps finished reading slot i -- have reached it.
+        // s_warp has two buffers by group parity. The readers below (2*S*cs threads: warps 0 AND 1 for
+        // S = 4, cs = 8) are ordered only before this CTA's own __syncthreads of group i + 1, not before
+        // the other warps' writes of group i + 1: the wait below completes on the send of whichever
+        // warp holds this CTA's own entries, so a warp may run into pass 1 of group i + 1 while the other
+        // reading warp still reads. Group i + 1 writes the other buffer; group i + 2 writes this one
+        // again only after the __syncthreads of group i + 1, which every reader of group i has reached.
         const uint32_t bar = smem_u32(&s_sum[q]);
         if (tid == 0) mbar_expect_tx(bar, sum_bytes);
         for (int e = tid; e < 2 * S * (int)cs; e += kBwdThreads) {
             const int v = e % (2 * S), dst = e / (2 * S);
             float a = 0.f;
 #pragma unroll
-            for (int ww = 0; ww < kBwdThreads / 32; ++ww) a += s_warp[ww][v];
+            for (int ww = 0; ww < kBwdThreads / 32; ++ww) a += s_warp[i & 1][ww][v];
             st_async_f32(map_to_rank(smem_u32(&s_peer[q][rank][v]), (uint32_t)dst), a, map_to_rank(bar, (uint32_t)dst));
         }
         mbar_wait(bar, (uint32_t)(i / kSumSlots) & 1u);
